@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - env-steps/s of the batched step hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one gca_step over one batch of 65,536 environments per GPU (SingleAircraft2Env,
@@ -22,6 +22,9 @@ intruders) and the finish (+ spawn phase).  Prints ONE JSON line (rank 0).
 --impl reference times the CPU oracle port alone, with the oracle library only (no libgca.so, no
 product package): the reference is Python and cannot travel to the GPU box; the port is pinned
 bit-exact to it by tests/test_oracle_golden.py.
+
+--dump-outputs DIR writes what the last timed step returned (rank 0) as DIR/<name>.npy, so that two
+builds run with the same arguments (same seeds, same inputs) can be compared output for output.
 """
 import argparse
 import json
@@ -44,6 +47,7 @@ VARIANT = "SingleAircraft2Env"
 METRIC = "env_steps_per_sec"
 UNIT = "env-steps/s"
 GRAPH_STEPS = 50            # steps captured per CUDA graph (actions cycle through this many batches)
+DUMP_OBS_ROWS = 16384       # --dump-outputs: observation rows of a seeded sample of envs (21.5 MB of f32 at N = 80)
 
 
 def workload_name():
@@ -118,6 +122,17 @@ def bind_to_gpu_numa_node(index):
         return {"old": old, "note": "host thread and pinned buffers on NUMA node %d (%d cores) of GPU %s" % (node, len(use), bdf)}
     except Exception as e:     # no sysfs / no permission: leave the placement to the OS
         return {"old": None, "note": "not bound (%s)" % type(e).__name__}
+
+
+def dump_outputs(out_dir, env):
+    """What step() returned in the last timed step, as float32 (float64 where the output is) .npy files: reward, done
+    and info of every env, and obs of a fixed, seeded sample of envs whose ids obs_rows holds."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = np.sort(np.random.RandomState(0).choice(env.num_envs, min(DUMP_OBS_ROWS, env.num_envs), replace=False))
+    arrays = {"obs": env.obs.cpu().numpy()[rows], "obs_rows": rows.astype(np.float64), "reward": env.reward.cpu().numpy(),
+              "done": env.done.cpu().numpy(), "info": env.info.cpu().numpy()}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64 if a.dtype == np.float64 else np.float32))
 
 
 def restore_affinity(numa):
@@ -359,6 +374,8 @@ def main_gpu(args):
     stop.record()
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:              # before the legs below step the same envs again
+        dump_outputs(args.dump_outputs, env)
     ms = start.elapsed_time(stop)
     t = torch.tensor([ms], device="cuda", dtype=torch.float64)
     if world > 1:
@@ -897,7 +914,12 @@ def main():
     ap.add_argument("--steps", type=int, default=2000)
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl ours)")
     if args.impl == "reference":
         main_reference(args)
     else:

@@ -197,6 +197,31 @@ def bench_config_keys():
     return bench.workload_config().keys()
 
 
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: step()'s outputs as float .npy files under 64 MB, obs rows a fixed seeded sample."""
+    import types
+    import torch
+    import bench
+    B = bench.ENVS_PER_GPU
+    g = torch.Generator().manual_seed(0)
+    env = types.SimpleNamespace(num_envs=B, obs=torch.rand((B, 4 * bench.N_INTRUDERS + 8), generator=g),
+                                reward=torch.rand((B,), generator=g),
+                                done=torch.randint(0, 2, (B,), dtype=torch.uint8, generator=g),
+                                info=torch.randint(0, 6, (B,), dtype=torch.uint8, generator=g))
+    bench.dump_outputs(str(tmp_path / "a"), env)
+    bench.dump_outputs(str(tmp_path / "b"), env)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["done.npy", "info.npy", "obs.npy", "obs_rows.npy", "reward.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / n) for n in names) <= 64 << 20
+    d = {n[:-4]: np.load(tmp_path / "a" / n) for n in names}
+    assert all(a.dtype in (np.float32, np.float64) for a in d.values())
+    rows = d["obs_rows"].astype(np.int64)
+    assert np.array_equal(d["obs"], env.obs.numpy()[rows]) and len(np.unique(rows)) == len(rows)
+    for k in ("reward", "done", "info"):
+        assert np.array_equal(d[k], getattr(env, k).numpy().astype(np.float32))
+    assert all(np.array_equal(d[n[:-4]], np.load(tmp_path / "b" / n)) for n in names)
+
+
 def test_bench_algorithmic_bytes():
     import bench
     assert bench.algorithmic_bytes_per_env_step(80) == 40 * 80 + 12 + 159
