@@ -44,7 +44,6 @@ struct gca_env {
   uint32_t env_id0 = 0;
   DevState s{};
   int D = 0;
-  bool fc_valid = false;    // the forecast words describe the current state (forecast step, gca_step_fc.cuh)
   // host path (gca_step_host[_begin / _wait] / gca_reset_host): compute stream, download stream, two sets of
   // device-side buffers and the events that order them
   cudaStream_t stream = nullptr, copy_stream = nullptr;
@@ -278,22 +277,9 @@ int gca_create(const gca_config* cfg, int n_envs, int n_intruders, int mode, int
   if (!rc) rc = dev_alloc(e, &s.ev_gone, flag_plane_words(s));
   if (!rc) rc = dev_alloc(e, &s.ev_nmac, (size_t)s.T * 32);
   if (!rc) rc = dev_alloc(e, &s.ev_near, (size_t)s.T * 32);
-  if (!rc) rc = dev_alloc(e, &s.reset_list, (size_t)s.T * 32);
-  if (!rc) rc = dev_alloc(e, &s.reset_count, 1);
-  s.respawn_cap = 0;                                  // (respawn records live in shared memory: step_finish_kernel)
-  if (!rc) rc = dev_alloc(e, &s.respawn_list, 1);
-  if (!rc) rc = dev_alloc(e, &s.respawn_count, 1);
   if (!rc) rc = dev_alloc(e, &s.pre, (size_t)s.T * 32);
   if (!rc) rc = dev_alloc(e, &s.step_seq, 1);
   if (!rc) rc = dev_alloc(e, &s.error_flag, 1);
-  if (!rc) rc = dev_alloc(e, &s.exit_count, 1);
-  if (!rc) rc = dev_alloc(e, &s.head_sync, 2);
-  if (!rc && draws == GCA_DRAWS_PHILOX && n_intruders > 0) {
-    rc = dev_alloc(e, &s.fc_gone, 3 * flag_plane_words(s));
-    if (!rc) rc = dev_alloc(e, &s.fc_near, 3 * (size_t)s.T * 32);
-    if (!rc) rc = dev_alloc(e, &s.fc_vmax, (size_t)s.T * 32);
-    if (!rc) rc = dev_alloc(e, &s.fc_queue, 4 + 2 * (size_t)s.T * 32);
-  }
   if (!rc) rc = dev_alloc(e, &s.ivel, vel_plane_bytes(s));
   if (!rc) rc = dev_alloc(e, &s.cflag, flag_plane_words(s));
   if (!rc) rc = dev_alloc(e, &s.dflag, mode == GCA_MODE_FAITHFUL ? flag_plane_words(s) : 1);
@@ -344,7 +330,6 @@ int gca_set_config(gca_env* e, const gca_config* cfg) {
     return fail(GCA_ERR_STATE, "the handle was created without per-intruder (heading, speed) state");
   e->cfg = *cfg;
   e->k = derive(*cfg);
-  e->fc_valid = false;
   return GCA_OK;
 }
 
@@ -356,11 +341,6 @@ int gca_reset(gca_env* e, const uint8_t* mask, const gca_tape* tape, const gca_o
   StepArgs a = make_args(e, nullptr, tape, out, 0);
   a.mask = mask;
   GCA_CUDA(launch_reset(e->mode == GCA_MODE_FAITHFUL, e->draws == GCA_DRAWS_TAPE, a, (cudaStream_t)stream));
-  e->fc_valid = false;
-  if (forecast_step_applies(a, e->draws == GCA_DRAWS_TAPE)) {
-    GCA_CUDA(launch_forecast(e->mode == GCA_MODE_FAITHFUL, a, (cudaStream_t)stream));
-    e->fc_valid = true;
-  }
   return GCA_OK;
 }
 
@@ -385,12 +365,6 @@ int gca_step(gca_env* e, const void* actions, const gca_tape* tape, int auto_res
     }
     ev = evs;
   }
-  if (forecast_step_applies(a, e->draws == GCA_DRAWS_TAPE)) {
-    if (!e->fc_valid) GCA_CUDA(launch_forecast(e->mode == GCA_MODE_FAITHFUL, a, (cudaStream_t)stream));
-    e->fc_valid = true;
-  } else {
-    e->fc_valid = false;
-  }
   GCA_CUDA(launch_step(e->mode == GCA_MODE_FAITHFUL, e->draws == GCA_DRAWS_TAPE, a, (cudaStream_t)stream, ev));
   return GCA_OK;
 }
@@ -407,8 +381,6 @@ int gca_check(gca_env* e) {
   int flag = 0;
   GCA_CUDA(cudaMemcpy(&flag, e->s.error_flag, sizeof(int), cudaMemcpyDeviceToHost));
   if (flag & 1) return fail(GCA_ERR_STATE, "a streaming lane timed out waiting for its ownship record (step_intruders_kernel)");
-  if (flag & 2) return fail(GCA_ERR_STATE, "forecast step: a departure forecast disagreed with the advance (step_intruders_kernel)");
-  if (flag & 4) return fail(GCA_ERR_STATE, "forecast step: a conflict in an env that the head kernel did not classify as hot");
   return GCA_OK;
 }
 
@@ -661,7 +633,6 @@ int gca_set_state(gca_env* e, const gca_host_state* h) {
       if (h->ihs && s.ihs) hp.hs[ihs_index(s, b, (int)i)] = make_double2(h->ihs[2 * k], h->ihs[2 * k + 1]);
     }
   }
-  e->fc_valid = false;
   return hp.upload(s, faith);
 }
 

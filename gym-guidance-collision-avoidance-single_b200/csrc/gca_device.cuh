@@ -53,27 +53,13 @@ struct DevState {
   uint32_t* ev_gone;      // [T][Wd][32] bit i: intruder i left the map
   int* ev_nmac;           // [T*32] lowest intruder index inside the NMAC radius (INT_MAX: none)
   uint32_t* ev_near;      // [T*32] shaped_nearest, FAST: bits of the smallest squared ownship-intruder distance of the step
-  int* reset_list;        // [T*32] envs that finished in this step (PHILOX auto-reset), in arrival order
-  int* reset_count;       // [1]
-  uint32_t* respawn_list; // [respawn_cap] (env << 8 | intruder) of the intruders that left the map in this step (PHILOX)
-  int* respawn_count;     // [T] records of each tile's segment of respawn_list
-  int respawn_cap;
+  uint64_t align_pad;     // unused: see StepArgs::align_pad
   // PHILOX handles (two kernels per step, see gca_step.cu)
   double2* pre;           // [T*32] what the ownship role settled before the intruders were looked at: (reward candidate,
                           //        bits: info | done << 8) of wall / goal / default / max-steps - the finish takes it unless an
                           //        intruder event outranks it
   uint32_t* step_seq;     // [1] steps launched on this handle; own_b.w of step k carries stamp k + 1 (valid under graph replay)
-  int* error_flag;        // [1] bit 0: a streaming lane's ownship record never arrived (dispatch order broke); forecast step:
-                          //     bit 1: a departure forecast disagrees with the advance, bit 2: a conflict in an env not classified hot
-  // forecast step (gca_step_fc.cu): three slots rotating with the env's tick z - a step reads slot z % 3, fills slot
-  // (z + 1) % 3 and clears slot (z + 2) % 3
-  uint32_t* fc_gone;      // [3][T][Wd][32] bit i: intruder i leaves the map at its next advance
-  uint32_t* fc_near;      // [3][T*32] f32 bits of the smallest squared ownship-intruder distance of the current state
-  float* fc_vmax;         // [T*32] upper bound of the distance an intruder of the env covers per step
-  uint32_t* exit_count;   // [1] blocks of the streaming kernel that are done with this step
-  uint32_t* head_sync;    // [2] (blocks of the head kernel that are done with this step, stamp of the step whose head is complete)
-  int* fc_queue;          // [4 + 2 T*32] (hot envs, finished envs, job cursor, tail blocks done), then the two env lists:
-                          // the warp jobs of the tail kernel
+  int* error_flag;        // [1] 1: a streaming lane's ownship record never arrived (dispatch order broke)
   size_t pos_plane;       // bytes of one position plane
   int B, N, T, U, W, Wd;
 };
@@ -163,7 +149,9 @@ struct StepArgs {
   int D;                  // observation row length
   int auto_reset;
   int own_blocks;         // PHILOX: leading blocks of step_intruders_kernel that play the ownship role (0: TAPE, own kernel)
-  int head_ctas;          // forecast step: blocks of step_head_kernel (each owns every head_ctas-th group of 128 envs)
+  int align_pad;          // unused: with DevState::align_pad it keeps every field at the offset modulo 16 that the step
+                          // kernels were tuned with - the compiler fetches a 16-byte aligned pair of 8-byte fields from
+                          // the constant bank with one load, so shifting the fields by 8 bytes changes the kernels' code
   void* obs;
   void* achieved;
   void* desired;

@@ -7,12 +7,6 @@
 namespace gca {
 cudaError_t launch_step(bool faith, bool tape, const StepArgs& a, cudaStream_t st, cudaEvent_t* ev);
 int step_launch_count(bool tape, int n_intruders, int obs_kind, bool turns);
-// the forecast step (gca_step_fc.cu): head kernel + streaming role, nothing behind them
-bool forecast_step_applies(const StepArgs& a, bool tape);
-cudaError_t launch_step_fc(bool faith, const StepArgs& a, cudaStream_t st, cudaEvent_t* ev);
-cudaError_t launch_forecast(bool faith, const StepArgs& a, cudaStream_t st);
-cudaError_t launch_stream_fc(bool faith, const StepArgs& a, cudaStream_t st);
-cudaError_t launch_step_tail(bool faith, const StepArgs& a, cudaStream_t st);
 cudaError_t launch_reset(bool faith, bool tape, const StepArgs& a, cudaStream_t st);
 cudaError_t launch_observe(bool faith, const StepArgs& a, cudaStream_t st);
 cudaError_t launch_compute_reward(const void* ag, long long n_ag, const void* g, long long m, double radius, int kind,

@@ -30,7 +30,6 @@
 //                          what the ownship role settled), counters, the scalar part of the VecEnv auto-reset; and
 //                          in the same launch the spawn phase: one lane per respawn, one warp per 32 spawns of a
 //                          reset (tape handles respawn in place, in the reference's draw order).
-// The opt-in forecast step (GCA_FORECAST=1) lives in gca_step_fc.cuh.
 // Every byte of intruder state is read once and written once per step; nothing is staged in HBM except
 // 16 bytes per env (ownship position for the streaming pass) and the event words.
 #include <climits>
@@ -47,7 +46,7 @@ namespace gca {
 
 // Optional kernel-level timestamps (build with -DGCA_PHASE_TIMING): first block in / last block out per kernel.
 #ifdef GCA_PHASE_TIMING
-__device__ unsigned long long g_kstamp[16];  // [kernel][start, end], then single stamps
+__device__ unsigned long long g_kstamp[8];   // [kernel][start, end] x 3, then the streaming pass's first record wait: begun, record seen
 __device__ __forceinline__ unsigned long long gtime() {
   unsigned long long t;
   asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
@@ -68,7 +67,7 @@ extern "C" int gca_debug_lat(unsigned int* host, int clear) {
 extern "C" int gca_debug_kstamps(unsigned long long* host, int reset) {
   int rc = (int)cudaMemcpyFromSymbol(host, g_kstamp, sizeof(g_kstamp));
   if (reset) {
-    unsigned long long init[16] = {~0ull, 0, ~0ull, 0, ~0ull, 0, ~0ull, ~0ull, ~0ull, 0, ~0ull, 0, 0, 0, 0, 0};
+    unsigned long long init[8] = {~0ull, 0, ~0ull, 0, ~0ull, 0, ~0ull, ~0ull};
     rc |= (int)cudaMemcpyToSymbol(g_kstamp, init, sizeof(init));
   }
   return rc;
@@ -94,9 +93,6 @@ constexpr int kWarpsB = GCA_WARPS_B;              // work items per block of the
 // staging row of one lane: 8 intruders x 16 bytes of observation entries, plus 16 bytes so that the row stride is
 // an odd multiple of 16 (conflict-free 16-byte shared accesses across a quarter warp)
 constexpr uint32_t kObsRow = 16u * kChunkIntr + 16u;
-#ifndef PDL_EARLY
-#define PDL_EARLY 0
-#endif
 
 // reset(): PKG/SingleAircraftEnv.py:66-98 for env `env`, executed by the whole warp; positions go to `plane`.
 // PHILOX: lanes = intruders.  TAPE: lane `owner` replays the reference's sequential draw order.
@@ -226,26 +222,10 @@ __device__ __forceinline__ void own_update(const StepArgs& a, const size_t me, c
     }
     s.ev_nmac[me] = INT_MAX;
     if (c.shaped_nearest) s.ev_near[me] = 0x7f800000u;            // +inf
-    if (me == 0) *s.reset_count = 0;
   } else {
-    // _terminal_reward() below the intruder loop   :173-183 and the variant rows of SURVEY.md 8(a)
-    double reward;
-    int info, done = 0;
-    if (maxstep_hit) {
-      reward = 0.0; done = 1; info = GCA_INFO_MAXSTEPS;
-    } else if (c.wall_kind != GCA_WALL_NONE && !in_map_f32(k, pos.x, pos.y)) {
-      reward = c.r_wall; done = c.wall_kind == GCA_WALL_TERMINAL; info = GCA_INFO_WALL;
-    } else {
-      const double dg = dist_f64((double)pos.x, (double)pos.y, goal.x, goal.y);
-      if (dg < c.goal_radius) {
-        reward = c.r_goal; done = 1; info = GCA_INFO_GOAL;
-      } else {
-        reward = c.shaped_default ? ddiv_prepared(k, -dg, k.dv_shape, k.rc_shape) : c.r_default;
-        info = GCA_INFO_NONE;
-      }
-    }
-    const double pre_bits = __longlong_as_double((long long)(info | (done << 8)));
-    stg_stream(&s.pre[me], make_float4(__int_as_float(__double2loint(reward)), __int_as_float(__double2hiint(reward)),
+    const Settled own = settle_own(c, k, maxstep_hit, pos, goal);
+    const double pre_bits = __longlong_as_double((long long)(own.info | (own.done << 8)));
+    stg_stream(&s.pre[me], make_float4(__int_as_float(__double2loint(own.reward)), __int_as_float(__double2hiint(own.reward)),
                                        __int_as_float(__double2loint(pre_bits)), __int_as_float(__double2hiint(pre_bits))),
                l2_evict_last_policy());
     write_obs_own<FAITH>(a, me, pos.x, pos.y, vel.x, vel.y, false, hs.x, hs.y, goal.x, goal.y);   // :115-124
@@ -255,7 +235,6 @@ __device__ __forceinline__ void own_update(const StepArgs& a, const size_t me, c
 template <bool FAITH, bool TAPE>
 __global__ void __launch_bounds__(128) step_own_kernel(const StepArgs a) {
   const DevState& s = a.s;
-  if (PDL_EARLY) pdl_launch_dependents();
   pdl_wait();
   GCA_KSTAMP_IN(0);
   const size_t me = (size_t)blockIdx.x * 128 + threadIdx.x;
@@ -464,7 +443,7 @@ __device__ __forceinline__ void finish_tile(const StepArgs& a, const int tile, c
   // PHILOX: a respawn depends on nothing but (env, tick, intruder) and the ownship position, so the spawns
   // (FP64-heavy, 0-3 per env) are not done here, one lane per env, but queued for spawn_kernel, which runs one
   // lane per spawn over the whole batch.  The records go to the tile's own segment of the respawn list.
-  int job_mine = 0, job_off = 0, job_total = 0, job_base = 0;
+  int job_mine = 0, job_off = 0, job_total = 0;
   if constexpr (!TAPE) {
     if (compact) {
       if (replay) job_mine = __popc(wg[0]) + __popc(wg[1]) + __popc(wg[2]) + __popc(wg[3]);
@@ -477,7 +456,6 @@ __device__ __forceinline__ void finish_tile(const StepArgs& a, const int tile, c
       job_total = __shfl_sync(FULL, job_off, 31);
       job_off -= job_mine;
       // the records go to the warp's shared scratch: the spawn phase of the same kernel runs them one lane each
-      job_base = 0;
     }
     if (lane == 0) ws->n_jobs = job_total < kTileRespawnCap ? job_total : kTileRespawnCap;   // (0 when the spawns were made in place)
   }
@@ -511,17 +489,10 @@ __device__ __forceinline__ void finish_tile(const StepArgs& a, const int tile, c
       const int bits = (int)__double_as_longlong(pre.y);
       reward = pre.x; info = bits & 0xff; done = (bits >> 8) != 0;
       is_default = info == GCA_INFO_NONE;
-    } else if (c.wall_kind != GCA_WALL_NONE && !in_map_f32(k, pos.x, pos.y)) {
-      reward = c.r_wall; done = c.wall_kind == GCA_WALL_TERMINAL; info = GCA_INFO_WALL;
     } else {
-      const double dg = dist_f64((double)pos.x, (double)pos.y, goal.x, goal.y);
-      if (dg < c.goal_radius) {
-        reward = c.r_goal; done = true; info = GCA_INFO_GOAL;
-      } else {
-        reward = c.shaped_default ? ddiv_prepared(k, -dg, k.dv_shape, k.rc_shape) : c.r_default;
-        info = GCA_INFO_NONE;
-        is_default = true;
-      }
+      const Settled own = settle_own(c, k, false, pos, goal);
+      reward = own.reward; info = own.info; done = own.done != 0;
+      is_default = info == GCA_INFO_NONE;
     }
     if (is_default && c.shaped_nearest) {                  // :225-232 (NumPy 2 weak scalars: an f32 distance stays f32)
       const double thr = 3 * c.minimum_separation;
@@ -555,14 +526,14 @@ __device__ __forceinline__ void finish_tile(const StepArgs& a, const int tile, c
     if (compact && job_total > 0) {
       if (job_mine > 0) {
         uint32_t set64_own[kWordsAhead] = {0u, 0u, 0u, 0u};
-        int at = job_base + job_off;
+        int at = job_off;
 #pragma unroll
         for (int w = 0; w < kWordsAhead; ++w) {
           uint32_t rest = wg[w];
           while (rest) {
             const int j = __ffs(rest) - 1;
             rest &= rest - 1;
-            if (at < job_base + kTileRespawnCap) ws->list[at] = ((uint32_t)lane << 8) | (uint32_t)(w * 32 + j);
+            if (at < kTileRespawnCap) ws->list[at] = ((uint32_t)lane << 8) | (uint32_t)(w * 32 + j);
             else if (!(done && a.auto_reset)) respawn_own(w * 32 + j, set64_own[w]);   // (list full: > 4 respawns per env on average)
             ++at;
           }
@@ -731,7 +702,6 @@ template <bool FAITH, bool TAPE>
 __global__ void __launch_bounds__(128) step_finish_kernel(const __grid_constant__ StepArgs a) {
   __shared__ WarpScratch ws[TAPE ? 1 : 4];
   __shared__ BlockScratch bs;
-  if (PDL_EARLY) pdl_launch_dependents();
   if (!TAPE && threadIdx.x == 0) bs.count = 0;
   pdl_wait();
   GCA_KSTAMP_IN(2);
@@ -768,10 +738,6 @@ __global__ void __launch_bounds__(128, MINB) step_n0_kernel(const __grid_constan
   if (tile < a.s.T) finish_tile<FAITH, false>(a, (int)tile, lane, &ws[wib], &bs);   // (reads back what this thread stored)
 }
 
-}  // namespace gca
-#include "gca_step_fc.cuh"   // the forecast step: ownship role, jobs kernel, launch_step_fc (one translation unit: shared timing stamps)
-namespace gca {
-
 // ------------------------------------------------------------------------------ 2. intruders (the streaming pass)
 // OM: 1 = the observation is GCA_OBS_VECTOR with the one-correction division exact (the registered ids'
 // layout; FAST only): entries are computed without run-time layout tests and leave through the transposed
@@ -779,24 +745,10 @@ namespace gca {
 // entries start 24 bytes into the row: 8-byte stores.  0 = generic (any layout, both modes): per-lane stores.
 // DRIFT: every advance adds Config.position_sigma to the velocity (the random-intruder env); generic layout only, so the
 // instruction streams of the other instantiations are what they were without it.
-// FC: the streaming role of the forecast step (gca_step_fc.cu).  step_head_kernel, launched just before with a
-// programmatic launch edge, publishes the ownship records and - concurrently with this pass - replaces the intruders
-// that the previous step FORECAST to leave the map in this one, and advances whole envs itself where the reference's
-// sequential semantics can matter (a conflict is possible, or the env finishes and is reset).  This pass therefore
-// (i) stores nothing for an intruder whose forecast bit is set (the head writes its successor) and nothing at all for
-// an env whose record carries kOwnSkip, (ii) forecasts the departures of the NEXT step from the positions it stores
-// (the same f32 sum the next step will make) and (iii) keeps the smallest squared distance of the new state, from
-// which the next head decides which envs can possibly see a conflict.  Nothing runs after it.
-template <bool FAITH, int OM, bool DRIFT = false, bool FC = false>
-__global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : (FC ? 8 : 1)) step_intruders_kernel(const __grid_constant__ StepArgs a) {
+template <bool FAITH, int OM, bool DRIFT = false>
+__global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : 1) step_intruders_kernel(const __grid_constant__ StepArgs a) {
   static_assert(!(DRIFT && OM), "a handle with a position drift takes the generic observation path");
-  if constexpr (!FC) {
-    if (PDL_EARLY) pdl_launch_dependents();
-    pdl_wait();
-  } else {
-    pdl_wait();                                           // the previous step (its tail kernel closed it) is complete
-    pdl_launch_dependents();                              // the tail kernel may be scheduled once the last block of this grid is resident
-  }
+  pdl_wait();
   GCA_KSTAMP_IN(1);
 #ifdef GCA_PHASE_TIMING
   if (threadIdx.x == 0 && blockIdx.x < 8192) g_cta[2 * blockIdx.x] = gtime();
@@ -806,7 +758,7 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : (FC ? 8
   // observation staging: FAST specialised layouts 8 x 16 bytes per lane, FAITHFUL 8 x 32 bytes per lane (+ 16: odd stride)
   constexpr uint32_t kObsRow64 = 32u * kChunkIntr + 16u;
   constexpr uint32_t kWarpSmem = OM ? 32 * kObsRow : (FAITH ? 32 * kObsRow64 : 16);
-  constexpr uint32_t kStageBytes = (FC && kWarpsB * kWarpSmem < kJobCap * 4u) ? kJobCap * 4u : kWarpsB * kWarpSmem;   // (the head role's job list)
+  constexpr uint32_t kStageBytes = kWarpsB * kWarpSmem;
   __shared__ __align__(16) uint8_t stage_smem[kStageBytes];
   const DevState& s = a.s;
   const Derived& k = a.k;
@@ -814,15 +766,7 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : (FC ? 8
   // dispatched in index order, so every record a streaming lane waits for below belongs to a block that is already
   // running or done (the forward-progress argument of a decoupled look-back scan).
   uint32_t stamp = 0u;
-  bool head_block = false;
-  if constexpr (FC) {
-    stamp = *s.step_seq + 1u;
-    if (blockIdx.x < (unsigned)a.head_ctas) {               // the head role of the forecast step (gca_step_fc.cuh)
-      head_role_fc<FAITH>(a, stamp, reinterpret_cast<uint32_t*>(stage_smem));
-      head_block = true;
-    }
-  }
-  if (!FC && a.own_blocks > 0) {
+  if (a.own_blocks > 0) {
     stamp = *s.step_seq + 1u;
     if (blockIdx.x < (unsigned)a.own_blocks) {
       GCA_KSTAMP_IN(0);
@@ -839,13 +783,13 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : (FC ? 8
   }
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
   const int n_chunks = (s.U + kChunkUnits - 1) / kChunkUnits;
-  const long long work = (long long)(blockIdx.x - (unsigned)(FC ? a.head_ctas : a.own_blocks)) * kWarpsB + wib;
+  const long long work = (long long)(blockIdx.x - (unsigned)a.own_blocks) * kWarpsB + wib;
   do {                                                    // (one pass; `break` = this warp has no work item)
-  if (head_block || work >= (long long)s.T * n_chunks) break;
+  if (work >= (long long)s.T * n_chunks) break;
   // Philox handles walk the tiles forwards in even steps and backwards in odd ones: the plane this step reads is the
   // plane the previous step wrote, and what it wrote LAST is what is most likely still in the L2 (43.3 -> 42.6 us)
   const int tile_fwd = (int)(work / n_chunks), ch = (int)(work - (long long)tile_fwd * n_chunks);
-  const int tile = (!FC && a.own_blocks > 0 && (stamp & 1u)) ? s.T - 1 - tile_fwd : tile_fwd;
+  const int tile = (a.own_blocks > 0 && (stamp & 1u)) ? s.T - 1 - tile_fwd : tile_fwd;
   const size_t me = (size_t)tile * 32 + lane;
   const bool has_env = me < (size_t)s.B;
   const int u0 = ch * kChunkUnits, i0 = 2 * u0;
@@ -864,7 +808,7 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : (FC ? 8
   }
   float4 ob;
   GCA_KSTAMP_IN(3);                                       // (timing builds: first streaming block in / first record seen)
-  if (FC || a.own_blocks > 0) {
+  if (a.own_blocks > 0) {
     // wait for this step's ownship record of the lane's env: it is stored with one 16-byte store and read with one
     // 16-byte aligned vector load, both served from one sector - a matching stamp comes with its position
     int spins = 0;
@@ -887,16 +831,6 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : (FC ? 8
   const bool runs = (bits & kOwnRuns) != 0;               // false: the reference's loop never ran for this env (max steps)
   const int par = (bits & kOwnPlane) ? 1 : 0;
   const float ox = ob.x, oy = ob.y;
-  // forecast step: fcw bit j = intruder i0 + j leaves the map in this step and the head replaces it
-  const bool skip = FC && (bits & kOwnSkip) != 0u;
-  uint32_t fcw = 0u, fnext = 0u;
-  size_t fc_fi = 0, fc_next = 0;
-  if constexpr (FC) {
-    const uint32_t slot = (bits >> kOwnSlotShift) & 3u;
-    fc_fi = flag_index(s, me, i0 >> 5);
-    fc_next = (size_t)(slot == 2u ? 0u : slot + 1u);
-    if (runs && !skip) fcw = (s.fc_gone[(size_t)slot * flag_plane_words(s) + fc_fi] >> (i0 & 31)) & ((1u << n_here) - 1u);
-  }
   const size_t pos_off = (unit0 * kPosUnits * 32 + lane) * 16;
   const uint8_t* psrc = s.ipos + (size_t)par * s.pos_plane + pos_off;
   uint8_t* pdst = s.ipos + (size_t)(par ^ 1) * s.pos_plane + pos_off;
@@ -941,66 +875,28 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : (FC ? 8
         const float d0 = dist2_f32(ox, oy, np[g].x, np[g].y), d1 = dist2_f32(ox, oy, np[g].z, np[g].w);   // :151
         conf |= ((d0 < k.sep2_f ? 1u : 0u) | (d1 < k.sep2_f ? 2u : 0u)) << (2 * g);
         nmac |= ((d0 < k.nmac2_f ? 1u : 0u) | (d1 < k.nmac2_f ? 2u : 0u)) << (2 * g);
-        if constexpr (FC) {                                 // (a replaced intruder's distance is the head's business)
-          near2 = fminf(near2, fminf(((fcw >> (2 * g)) & 1u) ? near2 : d0, ((fcw >> (2 * g)) & 2u) ? near2 : d1));
-        } else {
-          near2 = fminf(near2, fminf(d0, d1));
-        }
-      }
-      if constexpr (FC) {
-        if (runs && !skip && (gone & ~fcw) != 0u) atomicOr(s.error_flag, 2);   // a departure that was not forecast: never
-        // (the other direction cannot be tested here: the head may already have stored the successor's velocity)
+        near2 = fminf(near2, fminf(d0, d1));
       }
       if (!runs) {                                          // nobody moves: carry the positions over
         gone = conf = nmac = 0;
 #pragma unroll
         for (int g = 0; g < kChunkUnits; ++g) np[g] = p[g];
-        if constexpr (FC) {
-          near2 = __uint_as_float(0x7f800000u);
-#pragma unroll
-          for (int g = 0; g < kChunkUnits; ++g)
-            near2 = fminf(near2, fminf(dist2_f32(ox, oy, p[g].x, p[g].y), dist2_f32(ox, oy, p[g].z, p[g].w)));
-        }
       }
-      if constexpr (FC) {
-        // the next step's departures: the sum and the test it will make on what is stored now
+      if (has_env) {
+        // plain store, no evict_first hint: the plane written now is the plane the NEXT step reads, and with the
+        // observation stream marked evict_first a good part of its 42 MB is still in the 126 MB L2 then
+        // (48.6 -> 44.9 us per step; keeping the velocities as well - plain or evict_last loads - pushes the
+        // positions out again and gives the gain back)
 #pragma unroll
-        for (int g = 0; g < kChunkUnits; ++g) {
-          float4 dv = vv[g];
-          if constexpr (DRIFT)
-            dv = make_float4(__fadd_rn(dv.x, k.drift_f), __fadd_rn(dv.y, k.drift_f), __fadd_rn(dv.z, k.drift_f),
-                             __fadd_rn(dv.w, k.drift_f));
-          const float qx0 = __fadd_rn(np[g].x, dv.x), qy0 = __fadd_rn(np[g].y, dv.y);
-          const float qx1 = __fadd_rn(np[g].z, dv.z), qy1 = __fadd_rn(np[g].w, dv.w);
-          const bool o0 = (__float_as_uint(qx0) > wbits) | (__float_as_uint(qy0) > hbits);
-          const bool o1 = (__float_as_uint(qx1) > wbits) | (__float_as_uint(qy1) > hbits);
-          fnext |= ((o0 ? 1u : 0u) | (o1 ? 2u : 0u)) << (2 * g);
-        }
-        fnext &= ~fcw;
+        for (int g = 0; g < kChunkUnits; ++g) *reinterpret_cast<float4*>(pdst + g * 512) = np[g];
       }
-      if (has_env && !skip) {
-#pragma unroll
-        for (int g = 0; g < kChunkUnits; ++g) {
-          const uint32_t pb = FC ? (fcw >> (2 * g)) & 3u : 0u;
-          if (pb == 0u) {
-            // plain store, no evict_first hint: the plane written now is the plane the NEXT step reads, and with the
-            // observation stream marked evict_first a good part of its 42 MB is still in the 126 MB L2 then
-            // (48.6 -> 44.9 us per step; keeping the velocities as well - plain or evict_last loads - pushes the
-            // positions out again and gives the gain back)
-            *reinterpret_cast<float4*>(pdst + g * 512) = np[g];
-          } else {                                          // (the head stores the replaced half)
-            if (!(pb & 1u)) stg_stream2(pdst + g * 512, np[g].x, np[g].y, pol);
-            if (!(pb & 2u)) stg_stream2(pdst + g * 512 + 8, np[g].z, np[g].w, pol);
-          }
-        }
-      }
-      // The plane just read is dead when nothing can put an intruder back where it was (auto-reset; the forecast step's
-      // jobs read it later): its lines - largely still dirty in the L2 from the step that wrote them - are DISCARDED
-      // instead of being written back to DRAM (44.9 -> 43.3 us per step).  Lanes 0, 8, 16, 24 each discard the 128 bytes
+      // The plane just read is dead when nothing can put an intruder back where it was (auto-reset): its lines -
+      // largely still dirty in the L2 from the step that wrote them - are DISCARDED instead of being written back to
+      // DRAM (44.9 -> 43.3 us per step).  Lanes 0, 8, 16, 24 each discard the 128 bytes
       // that they and their 7 neighbours loaded; every (tile, unit) line is read by this warp only; the address
       // carries a dependency on the loaded data so that the discard cannot overtake the loads.  The plane is written in
       // full by the next step (stream + spawn phase) before anything reads it again.
-      if (!FC && a.auto_reset && (lane & 7) == 0) {
+      if (a.auto_reset && (lane & 7) == 0) {
 #pragma unroll
         for (int g = 0; g < kChunkUnits; ++g) {
           const uint8_t* q = psrc + g * 512 + ((__float_as_uint(np[g].x) | __float_as_uint(np[g].w)) & 0u);
@@ -1017,7 +913,6 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : (FC ? 8
           row[2 * g] = obs_intruder_vec(k, np[g].x, np[g].y, vv[g].x, vv[g].y);
           row[2 * g + 1] = obs_intruder_vec(k, np[g].z, np[g].w, vv[g].z, vv[g].w);
         }
-        if constexpr (FC) *reinterpret_cast<uint32_t*>(row + kChunkIntr) = skip ? 0xffu : fcw;   // (the row's padding)
         __syncwarp();
         constexpr int kLanesPerEnv = kChunkIntr, kEnvsPerStore = 32 / kLanesPerEnv;
         const int sub = lane / kLanesPerEnv, chunk = lane % kLanesPerEnv;
@@ -1028,10 +923,7 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : (FC ? 8
 #pragma unroll
         for (int it = 0; it < kLanesPerEnv; ++it) {
           const float4 val = *reinterpret_cast<const float4*>(src + it * kEnvsPerStore * kObsRow);
-          bool keep = true;
-          if constexpr (FC)
-            keep = !((*reinterpret_cast<const uint32_t*>(stg + (sub + it * kEnvsPerStore) * kObsRow + 16 * kChunkIntr) >> chunk) & 1u);
-          if (keep && env_sub + kEnvsPerStore * it < (size_t)s.B) {
+          if (env_sub + kEnvsPerStore * it < (size_t)s.B) {
             if constexpr (OM == 1) {
               stg_stream(dst + it * dstep, val, pol);
             } else {
@@ -1049,14 +941,14 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : (FC ? 8
             }
           }
         }
-      } else if (has_env && !skip) {
+      } else if (has_env) {
 #pragma unroll
         for (int g = 0; g < kChunkUnits; ++g) {
           Intr<FAITH> n0, n1;
           n0.px = np[g].x; n0.py = np[g].y; n0.vx = vv[g].x; n0.vy = vv[g].y;
           n1.px = np[g].z; n1.py = np[g].w; n1.vx = vv[g].z; n1.vy = vv[g].w;
-          if (!((fcw >> (2 * g)) & 1u)) write_obs_intruder<FAITH>(a, obase, i0 + 2 * g, n0);
-          if (!((fcw >> (2 * g)) & 2u)) write_obs_intruder<FAITH>(a, obase, i0 + 2 * g + 1, n1);
+          write_obs_intruder<FAITH>(a, obase, i0 + 2 * g, n0);
+          write_obs_intruder<FAITH>(a, obase, i0 + 2 * g + 1, n1);
         }
       }
     }
@@ -1097,24 +989,13 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : (FC ? 8
           conf |= (lt_sep ? 1u : 0u) << j;
           nmac |= (lt_nmac ? 1u : 0u) << j;
         }
-        if constexpr (FC) {
-          if (!((fcw >> j) & 1u)) {
-            near2 = fminf(near2, dist2_f32(ox, oy, (float)it.px, (float)it.py));
-            Intr<FAITH> nx = it;
-            if (advance<FAITH, DRIFT>(k, nx)) fnext |= 1u << j;
-          }
-        }
-        if (has_env && !skip && !((fcw >> j) & 1u)) *reinterpret_cast<double2*>(pdst + j * 512) = make_double2(it.px, it.py);
+        if (has_env) *reinterpret_cast<double2*>(pdst + j * 512) = make_double2(it.px, it.py);
         if (stage) {
           double o0, o1, o2, o3;
           obs_intruder_entries<FAITH>(a, it, o0, o1, o2, o3);
           row[2 * j] = make_double2(o0, o1);
           row[2 * j + 1] = make_double2(o2, o3);
         }
-      }
-      if constexpr (FC) {
-        if (runs && !skip && (gone & ~fcw) != 0u) atomicOr(s.error_flag, 2);
-        if (stage) *reinterpret_cast<uint32_t*>(stg + lane * kObsRow64 + 32 * kChunkIntr) = skip ? 0xffu : fcw;   // (row padding)
       }
       if (stage) {
         __syncwarp();
@@ -1124,10 +1005,7 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : (FC ? 8
         for (int it2 = 0; it2 < 16; ++it2) {
           const int e = sub + 2 * it2;
           const size_t env_e = (size_t)tile * 32 + e;
-          bool keep = true;
-          if constexpr (FC)
-            keep = !((*reinterpret_cast<const uint32_t*>(stg + e * kObsRow64 + 32 * kChunkIntr) >> (piece >> 1)) & 1u);
-          if (keep && env_e < (size_t)s.B) {
+          if (env_e < (size_t)s.B) {
             const double2 val = *reinterpret_cast<const double2*>(stg + e * kObsRow64 + piece * 16);
             double* dst = reinterpret_cast<double*>(a.obs) + env_e * (size_t)a.D + row_off + 2 * (size_t)piece;
             *reinterpret_cast<double2*>(dst) = val;
@@ -1136,7 +1014,7 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : (FC ? 8
       }
     }
   }
-  if (!fast_done && has_env && !skip) {
+  if (!fast_done && has_env) {
     // ---- generic: FAITHFUL positions (f64-capable) and the ragged last work item of a tile
     uint32_t dw = 0;
     if constexpr (FAITH) dw = s.dflag[flag_index(s, me, i0 >> 5)] >> (i0 & 31);
@@ -1160,46 +1038,12 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : (FC ? 8
         gone |= (oob ? 1u : 0u) << j;
         conf |= (lt_sep ? 1u : 0u) << j;
         nmac |= (lt_nmac ? 1u : 0u) << j;
-        if constexpr (!FAITH && !FC) near2 = fminf(near2, dist2_f32(ox, oy, it.px, it.py));
-      }
-      if constexpr (FC) {
-        if ((fcw >> j) & 1u) continue;                        // the head stores its successor
-        near2 = fminf(near2, dist2_f32(ox, oy, (float)it.px, (float)it.py));
-        Intr<FAITH> nx = it;
-        if (advance<FAITH, DRIFT>(k, nx)) fnext |= 1u << j;
+        if constexpr (!FAITH) near2 = fminf(near2, dist2_f32(ox, oy, it.px, it.py));
       }
       if constexpr (FAITH) *reinterpret_cast<double2*>(pdst + j * 512) = make_double2(it.px, it.py);
       else *reinterpret_cast<float2*>(pdst + (j >> 1) * 512 + (j & 1) * 8) = make_float2(it.px, it.py);
       write_obs_intruder<FAITH>(a, obase, i, it);
     }
-    if constexpr (FC) {
-      if (runs && (gone & ~fcw) != 0u) atomicOr(s.error_flag, 2);
-    }
-  }
-  if constexpr (FC) {
-    // ---- the forecast of the next step and the distance summary of the new state; a conflict here would mean the
-    // head's classification let an env through that it had to advance itself: flagged, never expected
-    if (has_env && !skip) {
-      if (fnext) atomicOr(&s.fc_gone[fc_next * flag_plane_words(s) + fc_fi], fnext << (i0 & 31));
-      atomicMin(&s.fc_near[fc_next * ((size_t)s.T * 32) + me], __float_as_uint(near2));
-    }
-    // ---- conflicts (PKG/SingleAircraftEnv.py:157-163, :169-170).  An env that reaches this point cannot see an NMAC
-    // in this step (the head advances those itself), so the order of the reference's loop does not matter: any
-    // intruder inside minimum_separation makes the step's return (r_conflict, False, 'c') - the head wrote what the
-    // step returns otherwise BEFORE it published the record -, sets its flag (which never clears, Q8) and counts if
-    // the flag was False.  A replaced intruder's test is the head's (its operands may already be its successor's).
-    const uint32_t cbits = conf & ~fcw;
-    if (has_env && !skip && cbits) {
-      if (nmac & cbits) atomicOr(s.error_flag, 4);            // the head's classification let an NMAC through: never
-      reinterpret_cast<R*>(a.reward)[me] = (R)a.cfg.r_conflict;
-      a.info[me] = (uint8_t)GCA_INFO_CONFLICT;
-      const uint32_t fresh = (cbits << (i0 & 31)) & ~s.cflag[fc_fi];
-      if (fresh) {
-        atomicOr(&s.cflag[fc_fi], fresh);
-        atomicAdd(&s.counters[me].x, __popc(fresh));
-      }
-    }
-    break;
   }
   // ---- record the (rare) events; i0 is a multiple of 8, so the 8 bits never straddle a word
   if (has_env) {
@@ -1428,50 +1272,8 @@ static unsigned turn_blocks(const DevState& s) { return (unsigned)((size_t)s.T *
 // ev (nullable): 5 events recorded before / between / after the kernels of the step (gca_profile_*):
 //   TAPE    0 own 1 streaming 2 finish 3 (-) 4
 //   PHILOX  0 (-) 1 ownship role + streaming 2 finish + spawn phase 3 nearest / turn pass 4
-// the streaming role of the forecast step (gca_step_fc.cu launches the head kernel right before it)
-cudaError_t launch_stream_fc(bool faith, const StepArgs& a, cudaStream_t st) {
-  const DevState& s = a.s;
-  static bool once = false;
-  if (!once) {
-    prefer_carveout(step_intruders_kernel<true, 0, true, true>);
-    prefer_carveout(step_intruders_kernel<true, 0, false, true>);
-    prefer_carveout(step_intruders_kernel<false, 1, false, true>);
-    prefer_carveout(step_intruders_kernel<false, 2, false, true>);
-    prefer_carveout(step_intruders_kernel<false, 0, true, true>);
-    prefer_carveout(step_intruders_kernel<false, 0, false, true>);
-    once = true;
-  }
-  const int n_chunks = (s.U + kChunkUnits - 1) / kChunkUnits;
-  const unsigned blocks = (unsigned)(((long long)s.T * n_chunks + kWarpsB - 1) / kWarpsB) + (unsigned)a.head_ctas;
-  if (faith) {
-    if (a.k.has_drift) return launch_pdl(step_intruders_kernel<true, 0, true, true>, blocks, kWarpsB * 32, st, a);
-    return launch_pdl(step_intruders_kernel<true, 0, false, true>, blocks, kWarpsB * 32, st, a);
-  }
-  const bool own_first = a.cfg.obs_kind == GCA_OBS_HER || a.cfg.obs_kind == GCA_OBS_DHER;
-  const bool special = a.k.div1_ok && !a.k.has_drift;
-  if (special && a.cfg.obs_kind == GCA_OBS_VECTOR) return launch_pdl(step_intruders_kernel<false, 1, false, true>, blocks, kWarpsB * 32, st, a);
-  if (special && own_first) return launch_pdl(step_intruders_kernel<false, 2, false, true>, blocks, kWarpsB * 32, st, a);
-  if (a.k.has_drift) return launch_pdl(step_intruders_kernel<false, 0, true, true>, blocks, kWarpsB * 32, st, a);
-  return launch_pdl(step_intruders_kernel<false, 0, false, true>, blocks, kWarpsB * 32, st, a);
-}
-
-// the passes that need the FINAL intruder set of the step (PHILOX handles)
-cudaError_t launch_step_tail(bool faith, const StepArgs& a, cudaStream_t st) {
-  const DevState& s = a.s;
-  if (a.cfg.obs_kind == GCA_OBS_NEAREST) {
-    if (faith) launch_pdl(nearest_obs_kernel<true>, (unsigned)(((size_t)s.B + 31) / 32), 128, st, a);
-    else launch_pdl(nearest_obs_kernel<false>, (unsigned)(((size_t)s.B + 31) / 32), 128, st, a);
-  }
-  if (has_turn_pass(a)) {
-    if (faith) launch_pdl(turn_obs_kernel<true, true>, turn_blocks(s), 128, st, a);
-    else launch_pdl(turn_obs_kernel<false, true>, turn_blocks(s), 128, st, a);
-  }
-  return cudaGetLastError();
-}
-
 template <bool FAITH, bool TAPE>
 static cudaError_t launch_step_t(const StepArgs& a0, cudaStream_t st, cudaEvent_t* ev) {
-  if (forecast_step_applies(a0, TAPE)) return launch_step_fc(FAITH, a0, st, ev);
   StepArgs a = a0;
   const DevState& s = a.s;
   const unsigned env_blocks = (unsigned)(((size_t)s.T * 32 + 127) / 128);

@@ -1,4 +1,4 @@
-// gca_step_common.cuh - helpers shared by the step kernels of gca_step.cu and gca_step_fc.cu (sm_100a).
+// gca_step_common.cuh - helpers of the step kernels in gca_step.cu (sm_100a).
 #pragma once
 #include <cstdlib>
 #include <utility>
@@ -10,16 +10,10 @@ namespace gca {
 // bits of own_b.z (the ownship record the streaming pass reads)
 constexpr uint32_t kOwnRuns = 1u;       // the reference's intruder loop runs for this env in this step
 constexpr uint32_t kOwnPlane = 2u;      // parity of the env's current position plane
-constexpr uint32_t kOwnSkip = 4u;       // forecast step: another role advances this env (hot / resetting): the lane does nothing
-constexpr uint32_t kOwnSlotShift = 3u;  // forecast step: bits 3-4 = tick % 3, the forecast slot this step reads
-constexpr uint32_t kOwnConf = 32u;      // forecast step: an intruder can be inside minimum_separation after this step
-constexpr uint32_t kOwnHot = 64u;       // forecast step: class of the env for the jobs kernel - a warp replays the reference's loop
-constexpr uint32_t kOwnReset = 128u;    //                                                   - the env finished: reset()'s spawns
 
 // Programmatic dependent launch: the kernels of a step are launched with programmatic stream serialization, so
 // the next grid is staged (and its blocks scheduled as slots free up) while the current one drains.  A kernel
 // calls pdl_wait() before it touches anything an earlier kernel of the stream wrote.
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
 // ownship state right after reset: (50, 50), min speed, heading pi/4 (PKG/SingleAircraftEnv.py:72-76), or with
@@ -56,9 +50,32 @@ __device__ __forceinline__ Draws<TAPE> make_draws(const StepArgs& a, size_t me, 
   return d;
 }
 
-__device__ __forceinline__ void st_release_pair(float* p, float x, float y) {
-  asm volatile("st.volatile.global.v2.f32 [%0], {%1, %2};" ::"l"(p), "f"(x), "f"(y) : "memory");
+// what _terminal_reward() returns when no intruder event outranks it: max steps / wall / goal / default
+// (PKG/SingleAircraftEnv.py:173-183 and the variant rows of SURVEY.md 8(a))
+struct Settled {
+  double reward;
+  int info;
+  int done;
+};
+__device__ __forceinline__ Settled settle_own(const gca_config& c, const Derived& k, bool maxstep_hit, float2 pos, double2 goal) {
+  double reward;
+  int info, done = 0;
+  if (maxstep_hit) {
+    reward = 0.0; done = 1; info = GCA_INFO_MAXSTEPS;
+  } else if (c.wall_kind != GCA_WALL_NONE && !in_map_f32(k, pos.x, pos.y)) {
+    reward = c.r_wall; done = c.wall_kind == GCA_WALL_TERMINAL; info = GCA_INFO_WALL;
+  } else {
+    const double dg = dist_f64((double)pos.x, (double)pos.y, goal.x, goal.y);
+    if (dg < c.goal_radius) {
+      reward = c.r_goal; done = 1; info = GCA_INFO_GOAL;
+    } else {
+      reward = c.shaped_default ? ddiv_prepared(k, -dg, k.dv_shape, k.rc_shape) : c.r_default;
+      info = GCA_INFO_NONE;
+    }
+  }
+  return Settled{reward, info, done};
 }
+
 __device__ __forceinline__ void st_release_quad(float* p, float x, float y, float z, float w) {
   asm volatile("st.volatile.global.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(x), "f"(y), "f"(z), "f"(w) : "memory");
 }
@@ -82,28 +99,6 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), unsigned blocks, unsigne
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = use_pdl ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
-}
-
-// Kernels that are meant to share SMs must agree on the L1 / shared-memory split: an SM only changes it when it is
-// idle, so blocks of a kernel that prefers another split wait until the resident kernel has left the SM (measured:
-// the streaming kernel started 21 us late behind a persistent head kernel with the default preference).
-inline int shared_carveout_percent() {
-  static const int pct = std::getenv("GCA_CARVEOUT") ? std::atoi(std::getenv("GCA_CARVEOUT")) : 72;   // 164 KB of 228 KB
-  return pct;
-}
-template <typename... KArgs>
-static void prefer_carveout(void (*kernel)(KArgs...)) {
-  cudaFuncSetAttribute(reinterpret_cast<const void*>(kernel), cudaFuncAttributePreferredSharedMemoryCarveout, shared_carveout_percent());
-}
-
-// plain stream-ordered launch (for kernels that do not call pdl_wait)
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_plain(void (*kernel)(KArgs...), unsigned blocks, unsigned threads, cudaStream_t st, Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(blocks);
-  cfg.blockDim = dim3(threads);
-  cfg.stream = st;
   return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 

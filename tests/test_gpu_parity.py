@@ -467,24 +467,6 @@ def test_random_configurations_bit_exact_vs_oracle(case):
     print(vk, mode, "W,H", W, H, "N", n, "B", B)
 
 
-@pytest.mark.gpu
-def test_forecast_step_bit_exact_vs_oracle_in_subprocess():
-    """The opt-in forecast step (GCA_FORECAST=1: head role + streaming pass side by side, tail kernel for hot envs and
-    resets, csrc/gca_step_fc.cuh) must give the same bits as the default step: the Philox rollouts against the oracle
-    and the full-size case, re-run in a subprocess with the switch set (it is read once per process)."""
-    import os
-    import subprocess
-    import sys
-    env = dict(os.environ, GCA_FORECAST="1")
-    here = os.path.abspath(__file__)
-    sel = ("test_philox_rollout_bit_exact_vs_oracle or test_full_size_bit_exact_vs_oracle or test_state_roundtrip or "
-           "test_long_rollout_with_explicit_masked_resets_vs_oracle or test_random_configurations_bit_exact_vs_oracle")
-    out = subprocess.run([sys.executable, "-m", "pytest", here, "-x", "-q", "-m", "gpu", "-k", sel, "-p", "no:cacheprovider"],
-                         env=env, capture_output=True, text=True, timeout=900)
-    assert out.returncode == 0, out.stdout[-3000:] + out.stderr[-2000:]
-    assert " passed" in out.stdout
-
-
 def test_host_path_async_equals_device_path():
     """gca_step_host_begin / _wait (two steps in flight, double-buffered downloads) return, step for step, what the
     device-resident path returns for the same seed and actions; mixing in the synchronous gca_step_host keeps the order."""

@@ -30,7 +30,7 @@ env.reset()
 acts = [torch.rand((B, 2), device="cuda") * 2 - 1 for _ in range(8)]
 lib = abi.load()
 lib.gca_debug_kstamps.argtypes = [C.c_void_p, C.c_int]
-buf = np.zeros(16, np.uint64)
+buf = np.zeros(8, np.uint64)
 g1 = torch.cuda.CUDAGraph()
 side = torch.cuda.Stream()
 with torch.cuda.stream(side):
@@ -49,10 +49,9 @@ def show(st, label):
     t0 = int(min(st[0], st[2], st[4]))
     rel = lambda v: (int(v) - t0) / 1e3
     print(label)
-    print("  ownship kernel    first in %7.2f   last out %7.2f   first record out %7.2f   last record out %7.2f" % (rel(st[0]), rel(st[1]), rel(st[8]), rel(st[9])))
-    print("  jobs / finish     first in %7.2f   last out %7.2f   (respawns %d, hot envs %d, resets %d)" % (rel(st[4]), rel(st[5]), st[12], st[13], st[14]))
+    print("  ownship kernel    first in %7.2f   last out %7.2f" % (rel(st[0]), rel(st[1])))
+    print("  finish kernel     first in %7.2f   last out %7.2f" % (rel(st[4]), rel(st[5])))
     print("  streaming kernel  first in %7.2f   last out %7.2f   first record seen %7.2f" % (rel(st[2]), rel(st[3]), rel(st[7])))
-    print("  tail kernel       first in %7.2f   last out %7.2f" % (rel(st[10]), rel(st[11])))
 
 
 for rep in range(3):
@@ -62,7 +61,7 @@ for rep in range(3):
     torch.cuda.synchronize()
     lib.gca_debug_kstamps(buf.ctypes.data, 1)
     st = buf.astype(np.int64)
-    print("8-step graph: first in .. last out = %.2f us per step" % ((max(st[1], st[3], st[5], st[11]) - min(st[0], st[2], st[4])) / 8e3))
+    print("8-step graph: first in .. last out = %.2f us per step" % ((max(st[1], st[3], st[5]) - min(st[0], st[2], st[4])) / 8e3))
     g1.replay()
     torch.cuda.synchronize()
     lib.gca_debug_kstamps(buf.ctypes.data, 1)
@@ -82,21 +81,20 @@ for lo in edges:
     m = (end >= lo) & (end < lo + 4)
     if m.any():
         print("  t=%5.1f..%5.1f  blocks finished %5d  mean lifetime %.2f  resident at t %d" % (lo, lo + 4, m.sum(), (end - start)[m].mean(), ((start <= lo) & (end > lo)).sum()))
-# per-tile phases of the finish kernel (default step): start, loads, replay, reward + stores, reset + counters, spawn (i)
-if not os.environ.get("GCA_FORECAST"):
-    fb = np.zeros(2048 * 8, np.uint64)
-    lib.gca_debug_fin.argtypes = [C.c_void_p]
-    lib.gca_debug_fin(fb.ctypes.data)
-    f = fb.astype(np.int64).reshape(2048, 8)
-    f = f[f[:, 0] > 0]
-    dur = (f[:, 1] - f[:, 0]) / 1e3
-    print("finish_tile per tile (us): mean %.2f p50 %.2f p90 %.2f p99 %.2f max %.2f" % (dur.mean(), np.median(dur), np.percentile(dur, 90), np.percentile(dur, 99), dur.max()))
-    print("finish phases (us, mean): loads %.2f  replay %.2f  reward+stores %.2f  reset+counters %.2f  spawn phase (i) %.2f" % (
-        ((f[:, 4] - f[:, 0]) / 1e3).mean(), ((f[:, 5] - f[:, 4]) / 1e3).mean(), ((f[:, 6] - f[:, 5]) / 1e3).mean(),
-        ((f[:, 1] - f[:, 6]) / 1e3).mean(), ((f[:, 7] - f[:, 1]) / 1e3).mean()))
-    t0 = f[:, 0].min()
-    print("relative to the first finish warp: finish_tile starts p50 %.2f max %.2f; ends max %.2f; spawn (i) ends max %.2f" % (
-        (np.median(f[:, 0]) - t0) / 1e3, (f[:, 0].max() - t0) / 1e3, (f[:, 1].max() - t0) / 1e3, (f[:, 7].max() - t0) / 1e3))
+# per-tile phases of the finish kernel: start, loads, replay, reward + stores, reset + counters, spawn (i)
+fb = np.zeros(2048 * 8, np.uint64)
+lib.gca_debug_fin.argtypes = [C.c_void_p]
+lib.gca_debug_fin(fb.ctypes.data)
+f = fb.astype(np.int64).reshape(2048, 8)
+f = f[f[:, 0] > 0]
+dur = (f[:, 1] - f[:, 0]) / 1e3
+print("finish_tile per tile (us): mean %.2f p50 %.2f p90 %.2f p99 %.2f max %.2f" % (dur.mean(), np.median(dur), np.percentile(dur, 90), np.percentile(dur, 99), dur.max()))
+print("finish phases (us, mean): loads %.2f  replay %.2f  reward+stores %.2f  reset+counters %.2f  spawn phase (i) %.2f" % (
+    ((f[:, 4] - f[:, 0]) / 1e3).mean(), ((f[:, 5] - f[:, 4]) / 1e3).mean(), ((f[:, 6] - f[:, 5]) / 1e3).mean(),
+    ((f[:, 1] - f[:, 6]) / 1e3).mean(), ((f[:, 7] - f[:, 1]) / 1e3).mean()))
+t0 = f[:, 0].min()
+print("relative to the first finish warp: finish_tile starts p50 %.2f max %.2f; ends max %.2f; spawn (i) ends max %.2f" % (
+    (np.median(f[:, 0]) - t0) / 1e3, (f[:, 0].max() - t0) / 1e3, (f[:, 1].max() - t0) / 1e3, (f[:, 7].max() - t0) / 1e3))
 # position-load latency of the streaming pass (clock64 cycles from issue to data), by eighth of the walk order:
 # what the previous step wrote last is read first - L2 hits there show as a low-latency mode
 lb = np.zeros(8 * 64, np.uint32)
