@@ -745,4 +745,13 @@ __device__ __forceinline__ void write_obs_nearest(const StepArgs& a, size_t env,
   }
 }
 
+// The f32 bit pattern of the relabel reward: -(d > goal_radius).astype(np.float32) (PKG/SingleAircraftHEREnv.py:194-196),
+// -1.0 or -0.0, and (d < goal_radius).astype(np.float32) (PKG/SingleAircraftDiscreteHEREnv.py:184-186).  Selected and
+// stored as integers: ptxas (CUDA 12.9, sm_100a) turned `selp.f32 -0.0, -1.0` of the f32 kernels into an integer
+// select of 0 / -1 and an int-to-float conversion, which stores +0.0 where the reference returns -0.0.
+__device__ __forceinline__ uint32_t relabel_reward_bits(int kind, bool gt, bool lt) {
+  if (kind == GCA_OBS_HER) return gt ? 0xbf800000u : 0x80000000u;
+  return lt ? 0x3f800000u : 0u;
+}
+
 }  // namespace gca

@@ -107,7 +107,7 @@ __global__ void __launch_bounds__(256, GCA_HER_MINB) her_sample_kernel(const Her
         const float d = __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
         gt = d > (float)a.radius; lt = d < (float)a.radius;
       }
-      a.out_r[b] = a.kind == GCA_OBS_HER ? -(gt ? 1.0f : 0.0f) : (lt ? 1.0f : 0.0f);
+      reinterpret_cast<uint32_t*>(a.out_r)[b] = relabel_reward_bits(a.kind, gt, lt);
       if (a.out_e) a.out_e[b] = (int32_t)e;
       if (a.out_t) a.out_t[b] = t;
       if (a.out_ft) a.out_ft[b] = her ? ft : -1;

@@ -29,7 +29,7 @@ __global__ void __launch_bounds__(256) reward_kernel(const T2* __restrict__ ag, 
       gt = d > (float)radius;
       lt = d < (float)radius;
     }
-    out[i] = kind == GCA_OBS_HER ? -(gt ? 1.0f : 0.0f) : (lt ? 1.0f : 0.0f);
+    reinterpret_cast<uint32_t*>(out)[i] = relabel_reward_bits(kind, gt, lt);
   }
 }
 
