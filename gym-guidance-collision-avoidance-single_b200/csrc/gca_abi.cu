@@ -84,17 +84,6 @@ int dev_alloc(gca_env* e, T** p, size_t count) {
   return GCA_OK;
 }
 
-// smallest s with sqrt(s) >= thr, i.e. (sqrt(s) < thr) == (s < X); T = float or double
-template <typename T>
-T sq_threshold(T thr) {
-  if (!(thr > 0)) return 0;
-  T c = thr * thr;
-  const T inf = std::numeric_limits<T>::infinity();
-  while (c > 0 && std::sqrt(c) >= thr) c = std::nextafter(c, (T)0);
-  while (std::sqrt(c) < thr) c = std::nextafter(c, inf);
-  return c;
-}
-
 // cached exhaustive check that the one-correction division is exact for divisor d
 bool div1_exact(float d) {
   static std::mutex mu;

@@ -1,10 +1,25 @@
-// gca_launch.h - host-callable launchers of the kernels in gca_step.cu / gca_reward.cu.
+// gca_launch.h - host-callable launchers of the kernels, and the host helpers they share.
 #pragma once
 #include <cuda_runtime.h>
+
+#include <cmath>
+#include <limits>
 
 #include "gca_device.cuh"
 
 namespace gca {
+// smallest s with sqrt(s) >= thr, i.e. (sqrt(s) < thr) == (s < X); T = float or double
+template <typename T>
+T sq_threshold(T thr) {
+  if (!(thr > 0)) return 0;
+  T c = thr * thr;
+  const T inf = std::numeric_limits<T>::infinity();
+  while (c > 0 && std::sqrt(c) >= thr) c = std::nextafter(c, (T)0);
+  while (std::sqrt(c) < thr) c = std::nextafter(c, inf);
+  return c;
+}
+
+
 cudaError_t launch_step(bool faith, bool tape, const StepArgs& a, cudaStream_t st, cudaEvent_t* ev);
 int step_launch_count(bool tape, int n_intruders, int obs_kind, bool turns);
 cudaError_t launch_reset(bool faith, bool tape, const StepArgs& a, cudaStream_t st);

@@ -7,11 +7,13 @@
 // conflict and goal both use minimum_separation and there is no NMAC tier (Q24), the wall test
 // is strict (Q6).
 //
-// Three users of the model (details at each kernel):
-//   mcts_playout_shared_kernel  position_sigma == 0 (the reference's setting): one CTA per root, intruder trajectories
-//                               shared by the root's playouts, one playout per lane;
-//   mcts_playout_kernel<RC>     any sigma: one warp per playout (below);
-//   mcts_candidates_kernel + mcts_search_kernel   the whole UCT search of a root in one lane, trees resident in HBM.
+// Users of the model (details at each kernel):
+//   mcts_playout_packed_kernel      position_sigma == 0 (the reference's setting): intruder trajectories shared by a
+//                                   root's playouts, one playout per lane;
+//   mcts_playout_rnd_lane_kernel    the random-intruder model up to 80 intruders and 256 playouts: one playout per lane;
+//   mcts_playout_kernel<RC, RND>    every other playout launch: one warp per playout (below);
+//   mcts_candidates_kernel + mcts_search_kernel   the whole UCT search of a root in one lane, trees resident in HBM;
+//   mcts_move_kernel                one move() per state (the drop-in node classes, tape replay).
 //
 // playout kernel: one warp per playout.  What is sequential in the reference is split so that the
 // expensive f64 work runs lane-parallel:
@@ -25,8 +27,6 @@
 //       the loop ends at the first sub-frame with a wall / conflict / goal event.
 // The kernel is bound by the FP64 pipe (about 8 DFMA-class instructions per intruder per sub-frame),
 // not by HBM: a root state (2.6 KB at N = 80) is read once per playout and stays in registers.
-#include <cstdlib>
-
 #include <algorithm>
 #include "gca_launch.h"
 
@@ -110,6 +110,63 @@ __device__ __forceinline__ double shfl_f64(double v, int src) {
   return __shfl_sync(FULL, v, src);
 }
 
+// the action of a playout's move at `depth`: the caller's first action where one is given (>= 0), else rollout_policy's
+__device__ __forceinline__ int playout_action(const MctsArgs& a, long long pid, uint32_t root, uint32_t playout, int depth) {
+  if (depth == 0 && a.first_action && a.first_action[pid] >= 0) return a.first_action[pid];
+  return mcts_action(a, root, playout, (uint32_t)depth);
+}
+
+__device__ __forceinline__ double lane_reward(int flags, double ox, double oy, double gx, double gy) {
+  if (flags & (GCA_MCTS_WALL | GCA_MCTS_CONFLICT)) return 0.0;
+  if (flags & GCA_MCTS_GOAL) return 1.0;
+  const double dx = __dadd_rn(ox, -gx), dy = __dadd_rn(oy, -gy);
+  const double dist = __dsqrt_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
+  return __dadd_rn(1.0, -__ddiv_rn(dist, 1200.0));
+}
+
+__device__ __forceinline__ void store_playout(const MctsArgs& a, long long pid, int first, int flags, double reward) {
+  a.rewards[pid] = reward;
+  if (a.first_out) a.first_out[pid] = (int8_t)first;
+  if (a.flags) a.flags[pid] = (uint8_t)flags;
+}
+
+// The random-intruder model (nodes_single_randintru.py) without position / speed noise (a.cull): every aircraft moves at
+// most its speed per sub-frame (an intruder: its root velocity until it first turns, then `speed` along its heading; the
+// ownship: clamp(...) <= max_speed).  An intruder further away at the root than both reaches plus the separation radius
+// can never raise the conflict flag in the playout, and nothing else of it is observable (reward and flags are the only
+// outputs): it is dropped.  The survivors keep their index - the draws of intruder i are addressed by i - so the playout
+// is bit-identical to the one that simulates all N (what the oracle does); typically ~10 of 80 remain.
+// One warp: the six entries of the kept intruders of root state st (ownship entries at own) go to dst, their indices to
+// idx; returns how many.  Without a.cull every intruder is kept.
+__device__ __forceinline__ int cull_intruders(const MctsArgs& a, const double* st, const double* own, int lane, double* dst,
+                                              int* idx) {
+  const gca_mcts_config& c = a.c;
+  const double frames = (double)a.depth * (double)c.simulate_frame;
+  const double own_reach = fmax(fabs(c.max_speed), fabs(c.min_speed)) * frames;
+  int n_eff = 0;
+  for (int base = 0; base < a.near; base += 32) {
+    const int i = base + lane;
+    double v[6] = {0., 0., 0., 0., 0., 0.};
+    bool keep = false;
+    if (i < a.near) {
+#pragma unroll
+      for (int q = 0; q < 6; ++q) v[q] = st[6 * i + q];
+      const double dx = v[0] - own[0], dy = v[1] - own[1];
+      const double reach = fmax(sqrt(v[2] * v[2] + v[3] * v[3]), fabs(v[4])) * frames;
+      keep = !a.cull || !(sqrt(dx * dx + dy * dy) > own_reach + reach + c.minimum_separation + 2.0);   // (NaN: kept)
+    }
+    const uint32_t mask = __ballot_sync(FULL, keep);
+    const int at = n_eff + __popc(mask & ((1u << lane) - 1u));
+    if (keep) {
+#pragma unroll
+      for (int q = 0; q < 6; ++q) dst[6 * at + q] = v[q];
+      idx[at] = i;
+    }
+    n_eff += __popc(mask);
+  }
+  return n_eff;
+}
+
 constexpr int kMctsWarps = 4;
 constexpr int kMaxRounds = 4;       // intruder rounds held in registers (N - 1 <= 128); larger N uses the generic path
 static_assert(kMaxRounds == 4, "launch_mcts_playouts dispatches on 1..4 rounds");
@@ -152,35 +209,7 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_playout_kernel(const Mct
       ix[r] = p.x; iy[r] = p.y; ivx[r] = w.x; ivy[r] = w.y;
     }
   } else if constexpr (RND) {
-    // Without position / speed noise every aircraft moves at most its speed per sub-frame (an intruder: its root
-    // velocity until it first turns, then `speed` along its heading; the ownship: clamp(...) <= max_speed).  An
-    // intruder further away at the root than both reaches plus the separation radius can never raise the conflict
-    // flag in this playout, and nothing else of it is observable (reward and flags are the only outputs): it is
-    // dropped.  The survivors keep their index - the draws of intruder i are addressed by i - so the playout is
-    // bit-identical to the one that simulates all N (what the oracle does); typically ~10 of 80 remain.
-    const double frames = (double)a.depth * (double)c.simulate_frame;
-    const double own_reach = fmax(fabs(c.max_speed), fabs(c.min_speed)) * frames;
-    n_eff = 0;
-    for (int base = 0; base < a.near; base += 32) {
-      const int i = base + lane;
-      double v[6] = {0., 0., 0., 0., 0., 0.};
-      bool keep = false;
-      if (i < a.near) {
-#pragma unroll
-        for (int q = 0; q < 6; ++q) v[q] = st[6 * i + q];
-        const double dx = v[0] - own[0], dy = v[1] - own[1];
-        const double reach = fmax(sqrt(v[2] * v[2] + v[3] * v[3]), fabs(v[4])) * frames;
-        keep = !a.cull || !(sqrt(dx * dx + dy * dy) > own_reach + reach + c.minimum_separation + 2.0);   // (NaN: kept)
-      }
-      const uint32_t mask = __ballot_sync(FULL, keep);
-      const int at = n_eff + __popc(mask & ((1u << lane) - 1u));
-      if (keep) {
-#pragma unroll
-        for (int q = 0; q < 6; ++q) sm[6 * at + q] = v[q];
-        sidx[at] = i;
-      }
-      n_eff += __popc(mask);
-    }
+    n_eff = cull_intruders(a, st, own, lane, sm, sidx);
     __syncwarp();
   } else {
     for (int j = lane; j < PER * a.near; j += 32) sm[j] = st[j];
@@ -195,9 +224,7 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_playout_kernel(const Mct
   int depth = 0;
   // ---- one move() per iteration; sub-frames handled in chunks of 32 lanes
   while (!(flags || depth == a.depth)) {
-    int act;
-    if (depth == 0 && a.first_action && a.first_action[pid] >= 0) act = a.first_action[pid];
-    else act = mcts_action(a, root, playout, (uint32_t)depth);
+    const int act = playout_action(a, pid, root, playout, depth);
     if (first < 0) first = act;
     const double d_heading = __dmul_rn((double)(act / 3 - 1), c.d_heading);
     const double accel = __dmul_rn((double)(act % 3 - 1), c.d_speed);
@@ -303,113 +330,45 @@ __global__ void __launch_bounds__(kMctsWarps * 32) mcts_playout_kernel(const Mct
     }
     ++depth;
   }
-  if (lane == 0) {
-    double reward;
-    if (flags & (GCA_MCTS_WALL | GCA_MCTS_CONFLICT)) reward = 0.0;
-    else if (flags & GCA_MCTS_GOAL) reward = 1.0;
-    else {
-      const double dx = __dadd_rn(ox, -gx), dy = __dadd_rn(oy, -gy);
-      const double dist = __dsqrt_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
-      reward = __dadd_rn(1.0, -__ddiv_rn(dist, 1200.0));
-    }
-    a.rewards[pid] = reward;
-    if (a.first_out) a.first_out[pid] = (int8_t)first;
-    if (a.flags) a.flags[pid] = (uint8_t)flags;
-  }
+  if (lane == 0) store_playout(a, pid, first, flags, lane_reward(flags, ox, oy, gx, gy));
 }
 
 // ---- position_sigma == 0 (config_single.py:27, the reference's setting): the intruders of the model move on
 // trajectories that depend on nothing but the root - x_f = x_{f-1} + (vx + 0.0), the same f64 additions for every
-// playout of that root - and the ownship cannot move further than (f + 1) * max_speed from its root position by
-// sub-frame f when speed_sigma == 0 (speed = clamp(vy) in [min_speed, max_speed], Q23).  So, one CTA per root:
-//   phase 1 (thread = intruder): advance every intruder through all depth * simulate_frame sub-frames with the
-//           reference's additions and, per sub-frame, list (exact f64 position) those the ownship could reach;
-//   phase 2 (thread = playout): the whole playout runs in one lane - Philox / Box-Muller / sincos per sub-frame in
-//           the reference's order, wall test, exact distance test against the sub-frame's candidates only
-//           (uniform shared-memory reads), goal test - with no shuffles and no idle lanes in the scalar part.
-// Same arithmetic per playout as mcts_playout_kernel, so the results are bit-identical; about 14x fewer
-// instructions per playout at N = 80 (the 79 x 30 distance tests collapse to ~45).
-constexpr int kSharedThreads = 128;
+// playout of that root - and the ownship cannot move further than (gf + 1) * max_speed from its root position (ox0, oy0)
+// by global sub-frame gf when speed_sigma == 0 (speed = clamp(vy) in [min_speed, max_speed], Q23).  One sub-frame of an
+// intruder's trajectory: advances (x, y) through sub-frame gf and returns whether the ownship could reach it there (the
+// margins cover the rounding of the bound).
+__device__ __forceinline__ bool advance_in_reach(const gca_mcts_config& c, double ox0, double oy0, int gf, double vx,
+                                                 double vy, double& x, double& y) {
+  x = __dadd_rn(x, vx);
+  y = __dadd_rn(y, vy);
+  if (c.speed_sigma != 0.0) return true;
+  const double vmax = fmax(fabs(c.min_speed), fabs(c.max_speed));
+  const double reach = c.minimum_separation + (double)(gf + 1) * vmax * 1.000001 + 0.5;
+  const double dx = x - ox0, dy = y - oy0;
+  return !(dx * dx + dy * dy >= reach * reach);
+}
 
 // COMPACT: cnt[gf] .. cnt[gf + 1] delimit the sub-frame's candidates in one packed list (the search workspace);
-// otherwise cnt[gf] candidates at cand[gf * near] (the shared-memory layouts of the playout kernels)
+// otherwise cnt[gf] candidates at cand[gf * near] (the shared-memory layout of the packed playout kernel)
 template <bool COMPACT = false>
 __device__ __forceinline__ int lane_move(const MctsArgs& a, const int* __restrict__ cnt, const double2* __restrict__ cand,
                                          uint32_t root, uint32_t sim, int depth, int act, double gx, double gy,
                                          double& ox, double& oy, double& vy_prev, double& heading);
 
-__global__ void __launch_bounds__(kSharedThreads) mcts_playout_shared_kernel(const MctsArgs a) {
-  extern __shared__ __align__(16) uint8_t mcts_sh[];
-  const gca_mcts_config& c = a.c;
-  const int F = c.simulate_frame, TF = a.depth * F;
-  int* cnt = reinterpret_cast<int*>(mcts_sh);                                        // [TF]
-  double2* cand = reinterpret_cast<double2*>(mcts_sh + (((size_t)TF * 4 + 15) & ~(size_t)15));   // [TF][near]
-  const long long r_idx = blockIdx.x;
-  const uint32_t root = a.root_id0 + (uint32_t)r_idx;
-  const double* st = a.roots + r_idx * a.L;
-  const double* own = st + a.per * a.n;
-  const double ox0 = own[0], oy0 = own[1];
-  const double gx = own[6], gy = own[7];
-
-  for (int f = threadIdx.x; f < TF; f += kSharedThreads) cnt[f] = 0;
-  __syncthreads();
-  // ---- phase 1: intruder trajectories, candidates per sub-frame
-  {
-    const bool cull = c.speed_sigma == 0.0;
-    const double vmax = fmax(fabs(c.min_speed), fabs(c.max_speed));
-    for (int i = threadIdx.x; i < a.near; i += kSharedThreads) {
-      const double2 p0 = reinterpret_cast<const double2*>(st)[2 * i];
-      const double2 v0 = reinterpret_cast<const double2*>(st)[2 * i + 1];
-      double x = p0.x, y = p0.y;
-      const double vx = __dadd_rn(v0.x, 0.0), vy = __dadd_rn(v0.y, 0.0);     // vx + normal(0, 0) :54-57
-      for (int f = 0; f < TF; ++f) {
-        x = __dadd_rn(x, vx);
-        y = __dadd_rn(y, vy);
-        bool in = true;
-        if (cull) {
-          const double reach = c.minimum_separation + (double)(f + 1) * vmax * 1.000001 + 0.5;
-          const double dx = x - ox0, dy = y - oy0;
-          in = !(dx * dx + dy * dy >= reach * reach);
-        }
-        if (in) cand[(size_t)f * a.near + atomicAdd(&cnt[f], 1)] = make_double2(x, y);
-      }
-    }
-  }
-  __syncthreads();
-  // ---- phase 2: one playout per lane
-  for (int p = threadIdx.x; p < a.playouts; p += kSharedThreads) {
-    const long long pid = r_idx * a.playouts + p;
-    double ox = ox0, oy = oy0, vy_prev = own[3], heading = own[5];
-    int flags = 0, first = -1;
-    for (int depth = 0; depth < a.depth && !flags; ++depth) {
-      int act;
-      if (depth == 0 && a.first_action && a.first_action[pid] >= 0) act = a.first_action[pid];
-      else act = mcts_action(a, root, (uint32_t)p, (uint32_t)depth);
-      if (first < 0) first = act;
-      flags = lane_move(a, cnt, cand, root, (uint32_t)p, depth, act, gx, gy, ox, oy, vy_prev, heading);
-    }
-    double reward;
-    if (flags & (GCA_MCTS_WALL | GCA_MCTS_CONFLICT)) reward = 0.0;
-    else if (flags & GCA_MCTS_GOAL) reward = 1.0;
-    else {
-      const double dx = __dadd_rn(ox, -gx), dy = __dadd_rn(oy, -gy);
-      const double dist = __dsqrt_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
-      reward = __dadd_rn(1.0, -__ddiv_rn(dist, 1200.0));
-    }
-    a.rewards[pid] = reward;
-    if (a.first_out) a.first_out[pid] = (int8_t)first;
-    if (a.flags) a.flags[pid] = (uint8_t)flags;
-  }
-}
-
-// ---- the same, several roots per CTA and one depth at a time.  With one CTA per root the playouts of a root fill
-// 100 of 128 lanes (the fourth warp runs 4 lanes) and the [depth * simulate_frame][near] candidate array (38 KB at
-// N = 80) holds the CTA count per SM to five.  Here the lanes of a CTA are the playouts of R consecutive roots laid
-// end to end (4 roots x 100 playouts = 400 of 416 lanes), and the candidate lists exist for ONE depth at a time
-// (simulate_frame sub-frames: 12.8 KB per root at N = 80): per depth, phase 1 advances every intruder of the R roots
-// through the depth's sub-frames from where the previous depth left it (running position in shared memory, the same
-// chain of additions), then every lane runs its playout's move of that depth.  A lane's arithmetic is exactly that of
-// mcts_playout_shared_kernel - same results, bit for bit.
+// The lanes of a CTA are the playouts of R consecutive roots laid end to end (5 roots x 100 playouts = 500 of 512
+// lanes); a root with more than kPackThreads playouts runs alone (R = 1) in slices of kPackThreads playouts, a CTA per
+// slice (blockIdx.y), each slice rebuilding its root's candidate lists.  Per depth:
+//   phase 1 (thread = (root, intruder)): advance every intruder of the R roots through the depth's sub-frames from where
+//           the previous depth left it (running position in shared memory, the same chain of additions) and, per
+//           sub-frame, list (exact f64 position) those the ownship could reach;
+//   phase 2 (thread = playout): the playout's move of that depth runs in one lane - Philox / Box-Muller / sincos per
+//           sub-frame in the reference's order, wall test, exact distance test against the sub-frame's candidates only
+//           (uniform shared-memory reads), goal test - with no shuffles and no idle lanes in the scalar part.
+// Same arithmetic per playout as mcts_playout_kernel, so the results are bit-identical; at N = 80 the 79 x 30 distance
+// tests of a playout collapse to ~45.  The candidate lists exist for one depth at a time (simulate_frame sub-frames:
+// 12.8 KB per root at N = 80), so two CTAs fit an SM.
 constexpr int kPackThreads = 512;             // 2 CTAs x 512 threads x 64 registers fill the register file
 constexpr int kPackMaxRoots = 8;
 
@@ -423,8 +382,8 @@ __global__ void __launch_bounds__(kPackThreads, 2) mcts_playout_packed_kernel(co
   double2* cand = xs + (size_t)R * near;
   const long long r0 = (long long)blockIdx.x * R;
   const int r_here = (int)min((long long)R, a.n_roots - r0);
-  const int q = threadIdx.x, rl = q / a.playouts, p = q - rl * a.playouts;
-  const bool active = rl < r_here;
+  const int q = threadIdx.x, rl = q / a.playouts, p = q - rl * a.playouts + (int)(blockIdx.y * blockDim.x);
+  const bool active = rl < r_here && p < a.playouts;
   const long long r_idx = r0 + (active ? rl : 0);
   const uint32_t root = a.root_id0 + (uint32_t)r_idx;
   const double* own = a.roots + r_idx * a.L + a.per * a.n;
@@ -432,8 +391,6 @@ __global__ void __launch_bounds__(kPackThreads, 2) mcts_playout_packed_kernel(co
   const long long pid = r_idx * a.playouts + p;
   double ox = own[0], oy = own[1], vy_prev = own[3], heading = own[5];
   int flags = 0, first = -1;
-  const bool cull = c.speed_sigma == 0.0;
-  const double vmax = fmax(fabs(c.min_speed), fabs(c.max_speed));
   for (int depth = 0; depth < a.depth; ++depth) {
     for (int f = threadIdx.x; f < r_here * F; f += blockDim.x) cnt[f] = 0;
     __syncthreads();
@@ -448,43 +405,22 @@ __global__ void __launch_bounds__(kPackThreads, 2) mcts_playout_packed_kernel(co
       double x = pos.x, y = pos.y;
       const double vx = __dadd_rn(v0.x, 0.0), vy = __dadd_rn(v0.y, 0.0);     // vx + normal(0, 0) :54-57
       for (int f = 0; f < F; ++f) {
-        x = __dadd_rn(x, vx);
-        y = __dadd_rn(y, vy);
-        bool in = true;
-        if (cull) {
-          const double reach = c.minimum_separation + (double)(depth * F + f + 1) * vmax * 1.000001 + 0.5;
-          const double dx = x - ox0, dy = y - oy0;
-          in = !(dx * dx + dy * dy >= reach * reach);
-        }
-        if (in) cand[((size_t)jr * F + f) * near + atomicAdd(&cnt[jr * F + f], 1)] = make_double2(x, y);
+        if (advance_in_reach(c, ox0, oy0, depth * F + f, vx, vy, x, y))
+          cand[((size_t)jr * F + f) * near + atomicAdd(&cnt[jr * F + f], 1)] = make_double2(x, y);
       }
       xs[(size_t)jr * near + i] = make_double2(x, y);
     }
     __syncthreads();
     // ---- phase 2 of this depth: lane = playout (lane_move indexes the lists by global sub-frame: shift the bases)
     if (active && !flags) {
-      int act;
-      if (depth == 0 && a.first_action && a.first_action[pid] >= 0) act = a.first_action[pid];
-      else act = mcts_action(a, root, (uint32_t)p, (uint32_t)depth);
+      const int act = playout_action(a, pid, root, (uint32_t)p, depth);
       if (first < 0) first = act;
       flags = lane_move(a, cnt + (rl - depth) * F, cand + (ptrdiff_t)(rl - depth) * F * near, root, (uint32_t)p, depth, act, gx, gy,
                         ox, oy, vy_prev, heading);
     }
     __syncthreads();
   }
-  if (active) {
-    double reward;
-    if (flags & (GCA_MCTS_WALL | GCA_MCTS_CONFLICT)) reward = 0.0;
-    else if (flags & GCA_MCTS_GOAL) reward = 1.0;
-    else {
-      const double dx = __dadd_rn(ox, -gx), dy = __dadd_rn(oy, -gy);
-      const double dist = __dsqrt_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
-      reward = __dadd_rn(1.0, -__ddiv_rn(dist, 1200.0));
-    }
-    a.rewards[pid] = reward;
-    if (a.first_out) a.first_out[pid] = (int8_t)first;
-    if (a.flags) a.flags[pid] = (uint8_t)flags;
-  }
+  if (active) store_playout(a, pid, first, flags, lane_reward(flags, ox, oy, gx, gy));
 }
 
 // ---- the random-intruder model (nodes_single_randintru.py), one playout per LANE.  In mcts_playout_kernel<0, true> a
@@ -516,33 +452,10 @@ __global__ void __launch_bounds__(kLaneThreads, GCA_LANE_MINB) mcts_playout_rnd_
   const long long r0 = (long long)blockIdx.x * R;
   const int r_here = (int)min((long long)R, a.n_roots - r0);
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
-  // ---- cull, a warp per root (see mcts_playout_kernel for the bound)
-  const double frames = (double)a.depth * (double)F;
-  const double own_reach = fmax(fabs(c.max_speed), fabs(c.min_speed)) * frames;
+  // ---- cull, a warp per root
   for (int jr = wib; jr < r_here; jr += n_warps) {
     const double* st = a.roots + (r0 + jr) * a.L;
-    const double* jo = st + a.per * a.n;
-    int n_eff = 0;
-    for (int b0 = 0; b0 < near; b0 += 32) {
-      const int i = b0 + lane;
-      double v[6] = {0., 0., 0., 0., 0., 0.};
-      bool keep = false;
-      if (i < near) {
-#pragma unroll
-        for (int q = 0; q < 6; ++q) v[q] = st[6 * i + q];
-        const double dx = v[0] - jo[0], dy = v[1] - jo[1];
-        const double reach = fmax(sqrt(v[2] * v[2] + v[3] * v[3]), fabs(v[4])) * frames;
-        keep = !a.cull || !(sqrt(dx * dx + dy * dy) > own_reach + reach + c.minimum_separation + 2.0);   // (NaN: kept)
-      }
-      const uint32_t mask = __ballot_sync(FULL, keep);
-      const int at = n_eff + __popc(mask & ((1u << lane) - 1u));
-      if (keep) {
-#pragma unroll
-        for (int q = 0; q < 6; ++q) base[((size_t)jr * near + at) * 6 + q] = v[q];
-        sidx[jr * near + at] = i;
-      }
-      n_eff += __popc(mask);
-    }
+    const int n_eff = cull_intruders(a, st, st + a.per * a.n, lane, base + (size_t)jr * near * 6, sidx + jr * near);
     if (lane == 0) neff[jr] = n_eff;
   }
   __syncthreads();
@@ -576,9 +489,7 @@ __global__ void __launch_bounds__(kLaneThreads, GCA_LANE_MINB) mcts_playout_rnd_
   const double gx = own[6], gy = own[7];
   int flags = 0, first = -1;
   for (int depth = 0; depth < a.depth && !flags; ++depth) {
-    int act;
-    if (depth == 0 && a.first_action && a.first_action[pid] >= 0) act = a.first_action[pid];
-    else act = mcts_action(a, root, playout, (uint32_t)depth);
+    const int act = playout_action(a, pid, root, playout, depth);
     if (first < 0) first = act;
     const double d_heading = __dmul_rn((double)(act / 3 - 1), c.d_heading);
     const double accel = __dmul_rn((double)(act % 3 - 1), c.d_speed);
@@ -632,17 +543,7 @@ __global__ void __launch_bounds__(kLaneThreads, GCA_LANE_MINB) mcts_playout_rnd_
       if (__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)) < a.sep2) { flags = GCA_MCTS_GOAL; break; }
     }
   }
-  double reward;
-  if (flags & (GCA_MCTS_WALL | GCA_MCTS_CONFLICT)) reward = 0.0;
-  else if (flags & GCA_MCTS_GOAL) reward = 1.0;
-  else {
-    const double dx = __dadd_rn(ox, -gx), dy = __dadd_rn(oy, -gy);
-    const double dist = __dsqrt_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
-    reward = __dadd_rn(1.0, -__ddiv_rn(dist, 1200.0));
-  }
-  a.rewards[pid] = reward;
-  if (a.first_out) a.first_out[pid] = (int8_t)first;
-  if (a.flags) a.flags[pid] = (uint8_t)flags;
+  store_playout(a, pid, first, flags, lane_reward(flags, ox, oy, gx, gy));
 }
 
 // ------------------------------------------------------------------------------ device-resident UCT search
@@ -744,14 +645,6 @@ __device__ __forceinline__ int lane_move(const MctsArgs& a, const int* __restric
   return 0;
 }
 
-__device__ __forceinline__ double lane_reward(int flags, double ox, double oy, double gx, double gy) {
-  if (flags & (GCA_MCTS_WALL | GCA_MCTS_CONFLICT)) return 0.0;
-  if (flags & GCA_MCTS_GOAL) return 1.0;
-  const double dx = __dadd_rn(ox, -gx), dy = __dadd_rn(oy, -gy);
-  const double dist = __dsqrt_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
-  return __dadd_rn(1.0, -__ddiv_rn(dist, 1200.0));
-}
-
 // intruder trajectories of one root -> per-sub-frame candidate lists, PACKED: ends[0] = 0 and ends[f + 1] = end of
 // sub-frame f's candidates in `cand` (so ends[f] is where they start).  Two passes over the same deterministic
 // trajectories: count, exclusive scan, place.  Packed because the search reads them one LANE per root: with the
@@ -763,23 +656,13 @@ __device__ __forceinline__ void walk_candidates(const MctsArgs& a, const double*
   const gca_mcts_config& c = a.c;
   const double* own = st + a.per * a.n;
   const double ox0 = own[0], oy0 = own[1];
-  const bool cull = c.speed_sigma == 0.0;
-  const double vmax = fmax(fabs(c.min_speed), fabs(c.max_speed));
   for (int i = tid; i < a.near; i += nthreads) {
     const double2 p0 = reinterpret_cast<const double2*>(st)[2 * i];
     const double2 v0 = reinterpret_cast<const double2*>(st)[2 * i + 1];
     double x = p0.x, y = p0.y;
     const double vx = __dadd_rn(v0.x, 0.0), vy = __dadd_rn(v0.y, 0.0);       // vx + normal(0, 0) :54-57
     for (int f = 0; f < TF; ++f) {
-      x = __dadd_rn(x, vx);
-      y = __dadd_rn(y, vy);
-      bool in = true;
-      if (cull) {
-        const double reach = c.minimum_separation + (double)(f + 1) * vmax * 1.000001 + 0.5;
-        const double dx = x - ox0, dy = y - oy0;
-        in = !(dx * dx + dy * dy >= reach * reach);
-      }
-      if (in) {
+      if (advance_in_reach(c, ox0, oy0, f, vx, vy, x, y)) {
         const int at = atomicAdd(&ends[f + 1], 1);          // count, or (PLACE) the sub-frame's fill pointer
         if (PLACE) cand[at] = make_double2(x, y);
       }
@@ -992,18 +875,10 @@ __global__ void __launch_bounds__(128) mcts_move_kernel(const MctsArgs a) {
   if (tape) a.cursor[k] = cur;
 }
 
-static double sq_threshold_f64(double thr) {
-  if (!(thr > 0)) return 0;
-  double c = thr * thr;
-  while (c > 0 && sqrt(c) >= thr) c = nextafter(c, 0.0);
-  while (sqrt(c) < thr) c = nextafter(c, INFINITY);
-  return c;
-}
-
 static MctsArgs mcts_base(const gca_mcts_config* cfg, int n) {
   MctsArgs a{};
   a.c = *cfg;
-  a.sep2 = sq_threshold_f64(cfg->minimum_separation);
+  a.sep2 = sq_threshold<double>(cfg->minimum_separation);
   a.n = n;
   a.per = cfg->random_intruders ? 6 : 4;
   a.L = a.per * n + 8;
@@ -1021,14 +896,10 @@ cudaError_t launch_mcts_playouts(const gca_mcts_config* cfg, int n, const double
   a.rewards = rewards; a.first_out = first_out; a.flags = flags;
   const long long total = n_roots * playouts;
   if (total <= 0) return cudaSuccess;
-  // position_sigma == 0: root-cooperative kernel (intruder trajectories shared by the root's playouts)
-  const long long tf = (long long)depth * cfg->simulate_frame;
-  const size_t shared_smem = (((size_t)tf * 4 + 15) & ~(size_t)15) + sizeof(double2) * (size_t)tf * (size_t)a.near;
-  const unsigned pblocks = (unsigned)((total + kMctsWarps - 1) / kMctsWarps);
-  if (cfg->random_intruders) {                // every playout moves its own intruders: one warp per playout
-    const size_t smem = sizeof(double) * kMctsWarps * (6 * (size_t)a.near + ((size_t)a.near + 1) / 2);
-    a.cull = cfg->position_sigma == 0.0 && cfg->speed_sigma == 0.0 && !getenv("GCA_MCTS_NO_CULL");
-    if (a.near <= kLaneMaxNear && playouts <= kLaneThreads && !getenv("GCA_MCTS_WARP_KERNEL")) {
+  const unsigned blocks = (unsigned)((total + kMctsWarps - 1) / kMctsWarps);
+  if (cfg->random_intruders) {                // every playout moves its own intruders
+    a.cull = cfg->position_sigma == 0.0 && cfg->speed_sigma == 0.0;
+    if (a.near <= kLaneMaxNear && playouts <= kLaneThreads) {
       // one playout per lane, several roots per CTA (mcts_playout_rnd_lane_kernel)
       const int R = (int)std::min<long long>(std::min<long long>(kLaneMaxRoots, kLaneThreads / playouts), n_roots);
       const size_t lsm = (((size_t)(16 + (size_t)R * a.near) * 4 + 15) & ~(size_t)15) + sizeof(double) * 6 * (size_t)R * (size_t)a.near;
@@ -1038,32 +909,28 @@ cudaError_t launch_mcts_playouts(const gca_mcts_config* cfg, int n, const double
       mcts_playout_rnd_lane_kernel<<<(unsigned)((n_roots + R - 1) / R), threads, lsm, st>>>(a, R);
       return cudaGetLastError();
     }
+    const size_t smem = sizeof(double) * kMctsWarps * (6 * (size_t)a.near + ((size_t)a.near + 1) / 2);
     cudaError_t e = cudaFuncSetAttribute(mcts_playout_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    mcts_playout_kernel<0, true><<<pblocks, kMctsWarps * 32, smem, st>>>(a);
+    mcts_playout_kernel<0, true><<<blocks, kMctsWarps * 32, smem, st>>>(a);
     return cudaGetLastError();
   }
-  if (cfg->position_sigma == 0.0 && playouts <= kPackThreads && depth > 0 && !getenv("GCA_MCTS_WARP_KERNEL") && !getenv("GCA_MCTS_NO_PACK")) {
-    // several roots per CTA, candidate lists of one depth at a time (mcts_playout_packed_kernel)
+  if (cfg->position_sigma == 0.0) {
+    // intruder trajectories shared by a root's playouts: several roots per CTA, or one root in slices of kPackThreads
+    // playouts (mcts_playout_packed_kernel)
     const size_t F = (size_t)cfg->simulate_frame;
     auto pack_smem = [&](int r) { return (((size_t)r * F * 4 + 15) & ~(size_t)15) + sizeof(double2) * (size_t)r * (size_t)a.near * (1 + F); };
-    int R = (int)std::min<long long>(std::min<long long>(kPackMaxRoots, kPackThreads / playouts), n_roots);
+    int R = (int)std::min<long long>(std::min(kPackMaxRoots, std::max(1, kPackThreads / playouts)), n_roots);
     while (R > 1 && 2 * pack_smem(R) > 200 * 1024) --R;      // two CTAs per SM
-    if (pack_smem(R) <= 200 * 1024) {
-      const unsigned threads = (unsigned)(((long long)R * playouts + 31) / 32 * 32);
+    const unsigned slices = (unsigned)((playouts + kPackThreads - 1) / kPackThreads);
+    if (pack_smem(R) <= 200 * 1024 && slices <= 65535) {     // (65535: the largest gridDim.y)
+      const unsigned threads = (unsigned)((std::min((long long)R * playouts, (long long)kPackThreads) + 31) / 32 * 32);
       cudaError_t e = cudaFuncSetAttribute(mcts_playout_packed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pack_smem(R));
       if (e != cudaSuccess) return e;
-      mcts_playout_packed_kernel<<<(unsigned)((n_roots + R - 1) / R), threads, pack_smem(R), st>>>(a, R);
+      mcts_playout_packed_kernel<<<dim3((unsigned)((n_roots + R - 1) / R), slices), threads, pack_smem(R), st>>>(a, R);
       return cudaGetLastError();
     }
   }
-  if (cfg->position_sigma == 0.0 && shared_smem <= 160 * 1024 && !getenv("GCA_MCTS_WARP_KERNEL")) {
-    cudaError_t e = cudaFuncSetAttribute(mcts_playout_shared_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shared_smem);
-    if (e != cudaSuccess) return e;
-    mcts_playout_shared_kernel<<<(unsigned)n_roots, kSharedThreads, shared_smem, st>>>(a);
-    return cudaGetLastError();
-  }
-  const unsigned blocks = (unsigned)((total + kMctsWarps - 1) / kMctsWarps);
   const int rounds = (a.near + 31) / 32;
   switch (rounds) {
     case 0:

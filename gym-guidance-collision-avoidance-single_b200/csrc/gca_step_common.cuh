@@ -1,6 +1,5 @@
 // gca_step_common.cuh - helpers of the step kernels in gca_step.cu (sm_100a).
 #pragma once
-#include <cstdlib>
 #include <utility>
 
 #include "gca_device.cuh"
@@ -88,7 +87,6 @@ __device__ __forceinline__ float4 ld_volatile_f4(const float4* p) {
 // launch with programmatic stream serialization (see pdl_wait above)
 template <typename... KArgs, typename... Args>
 static cudaError_t launch_pdl(void (*kernel)(KArgs...), unsigned blocks, unsigned threads, cudaStream_t st, Args&&... args) {
-  static const int use_pdl = std::getenv("GCA_NO_PDL") ? 0 : 1;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(blocks);
   cfg.blockDim = dim3(threads);
@@ -98,7 +96,7 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), unsigned blocks, unsigne
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = use_pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 

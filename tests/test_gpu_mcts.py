@@ -46,11 +46,13 @@ def test_move_replays_reference(stem, n):
 
 @pytest.mark.parametrize("n,roots_n,playouts,depth,over", [
     (80, 64, 100, 3, {}), (3, 200, 50, 3, {}), (1, 50, 20, 2, {}), (0, 50, 20, 3, {}),
-    (200, 16, 30, 3, {}),                                   # generic (shared-memory) intruder path
+    (200, 16, 30, 3, {}),                                   # 200 intruders: 2 roots per CTA
     (80, 8, 10, 4, {"simulate_frame": 10}),                 # 40 sub-frames: two lane chunks
     (20, 32, 20, 3, {"speed_sigma": 0.05, "position_sigma": 0.3}),
     (80, 48, 40, 3, RND), (3, 100, 50, 3, RND), (1, 40, 20, 2, RND), (0, 20, 10, 3, RND),
     (33, 24, 20, 4, dict(RND, speed_sigma=0.05, position_sigma=0.3, turn_prob=0.5)),
+    (80, 21, 100, 3, RND),                                  # 2 roots per CTA, ragged last CTA
+    (5, 7, 30, 3, dict(RND, speed_sigma=0.05, position_sigma=0.3, turn_prob=0.5)),
 ])
 def test_playouts_bit_exact_vs_oracle(n, roots_n, playouts, depth, over):
     import torch
@@ -69,34 +71,31 @@ def test_playouts_bit_exact_vs_oracle(n, roots_n, playouts, depth, over):
     print("n=%d flags histogram" % n, np.bincount(want_fl.ravel(), minlength=5).tolist())
 
 
+NOISE = {"speed_sigma": 0.05, "position_sigma": 0.3}
+
+
 @pytest.mark.parametrize("n,roots_n,playouts,depth,over", [
-    (80, 48, 40, 3, {}), (200, 8, 12, 3, {}), (80, 6, 8, 4, {}),
-    (80, 21, 100, 3, RND), (5, 7, 30, 3, dict(RND, speed_sigma=0.05, position_sigma=0.3, turn_prob=0.5)),
+    (20, 16, 30, 3, NOISE), (50, 12, 30, 3, NOISE), (80, 12, 30, 3, NOISE), (120, 8, 20, 3, NOISE),
+    (200, 6, 20, 3, NOISE),
+    (100, 8, 40, 3, RND), (100, 6, 20, 3, dict(RND, **NOISE)), (80, 5, 300, 3, RND),
 ])
-def test_warp_per_playout_kernel_bit_exact(n, roots_n, playouts, depth, over, monkeypatch):
-    """position_sigma == 0 takes the root-cooperative kernel and the random-intruder model the lane-per-playout kernel;
-    the warp-per-playout kernels (any sigma, any N) must keep giving the same bits (GCA_MCTS_WARP_KERNEL forces them)."""
-    if over:
-        test_playouts_bit_exact_vs_oracle(n, roots_n, playouts, depth, over)     # (lane-per-playout kernel, ragged last CTA)
-    monkeypatch.setenv("GCA_MCTS_WARP_KERNEL", "1")
+def test_warp_per_playout_kernel_bit_exact(n, roots_n, playouts, depth, over):
+    """Position noise takes the warp-per-playout kernel: mcts_playout_kernel<1..4> for up to 32..128 intruders, <0>
+    beyond.  So does the random-intruder model with more than 80 intruders or more than 256 playouts per root
+    (mcts_playout_kernel<0, true>; culled without noise, as in the last case)."""
     test_playouts_bit_exact_vs_oracle(n, roots_n, playouts, depth, over)
 
 
-@pytest.mark.parametrize("n,roots_n,playouts,depth", [(80, 37, 100, 3), (3, 9, 50, 3), (80, 5, 500, 2)])
-def test_one_root_per_cta_kernel_bit_exact(n, roots_n, playouts, depth, monkeypatch):
-    """position_sigma == 0 packs several roots into a CTA (mcts_playout_packed_kernel; 37 roots = a ragged last CTA);
-    the one-root-per-CTA kernel (more than 448 playouts per root, or GCA_MCTS_NO_PACK) must give the same bits."""
+@pytest.mark.parametrize("n,roots_n,playouts,depth", [
+    (80, 37, 100, 3), (3, 9, 50, 3), (80, 5, 500, 2),
+    (80, 5, 1100, 2), (3, 4, 1008, 3),
+    (80, 9, 40, 0), (80, 3, 1100, 0),
+])
+def test_packed_kernel_bit_exact(n, roots_n, playouts, depth):
+    """position_sigma == 0 takes mcts_playout_packed_kernel: several roots per CTA (37 roots of 100 playouts = a ragged
+    last CTA), one root per CTA (500 playouts), one root in slices of 512 playouts (1100 = three slices, the last one
+    ragged), and depth 0 (the reward of the root state itself)."""
     test_playouts_bit_exact_vs_oracle(n, roots_n, playouts, depth, {})
-    monkeypatch.setenv("GCA_MCTS_NO_PACK", "1")
-    test_playouts_bit_exact_vs_oracle(n, roots_n, playouts, depth, {})
-
-
-def test_random_intruder_playouts_without_culling_bit_exact(monkeypatch):
-    """The random-intruder playout kernel drops the intruders that cannot reach the ownship within the playout (exact:
-    results are compared with the oracle, which simulates all of them, above); with the culling switched off
-    (GCA_MCTS_NO_CULL) the kernel must give the same bits."""
-    monkeypatch.setenv("GCA_MCTS_NO_CULL", "1")
-    test_playouts_bit_exact_vs_oracle(80, 24, 30, 3, RND)
 
 
 def _random_roots(n, roots_n, seed, six=False):

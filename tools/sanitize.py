@@ -81,20 +81,17 @@ roots = env.reset().clone()
 env.close()
 mcts.playouts(roots, 37, depth=3, cfg=cfg, seed=1)                  # packed kernel: 8 roots per CTA
 mcts.playouts(roots[:13], 100, depth=3, cfg=cfg, seed=1)            # 5 roots per CTA, ragged last CTA
-os.environ["GCA_MCTS_NO_PACK"] = "1"
-mcts.playouts(roots, 37, depth=3, cfg=cfg, seed=1)                  # one root per CTA
-del os.environ["GCA_MCTS_NO_PACK"]
-os.environ["GCA_MCTS_WARP_KERNEL"] = "1"
-mcts.playouts(roots, 11, depth=3, cfg=cfg, seed=1)
-del os.environ["GCA_MCTS_WARP_KERNEL"]
+mcts.playouts(roots[:3], 1100, depth=2, cfg=cfg, seed=1)            # slices of 512 playouts, ragged last slice
+mcts.playouts(roots[:5], 40, depth=0, cfg=cfg, seed=1)              # depth 0
+ncfg = abi.make_mcts_config(MctsConfig)
+ncfg.position_sigma, ncfg.speed_sigma = 0.3, 0.05
+mcts.playouts(roots, 11, depth=3, cfg=ncfg, seed=1)                 # position noise: warp-per-playout kernel
 mcts.search(roots, 60, 3, cfg=cfg, seed=4)
 mcts.move(roots.clone(), torch.randint(0, 9, (48,), device="cuda", dtype=torch.int32), cfg)
 rcfg = abi.make_mcts_config(MctsConfig, random_intruders=True)      # the nodes_single_randintru.py model
 mcts.playouts(rnd_roots, 9, depth=3, cfg=rcfg, seed=1)              # lane-per-playout kernel, 8 roots per CTA
 mcts.playouts(rnd_roots[:7], 100, depth=3, cfg=rcfg, seed=1)        # 2 roots per CTA, ragged last CTA
-os.environ["GCA_MCTS_WARP_KERNEL"] = "1"
-mcts.playouts(rnd_roots, 9, depth=3, cfg=rcfg, seed=1)              # warp-per-playout kernel
-del os.environ["GCA_MCTS_WARP_KERNEL"]
+mcts.playouts(rnd_roots[:3], 300, depth=3, cfg=rcfg, seed=1)        # more than 256 playouts: warp-per-playout kernel
 mcts.move(rnd_roots.clone(), torch.randint(0, 9, (24,), device="cuda", dtype=torch.int32), rcfg)
 torch.cuda.synchronize()
 print("ok mcts", flush=True)
