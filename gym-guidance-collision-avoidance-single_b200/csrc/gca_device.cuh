@@ -468,8 +468,7 @@ __device__ __forceinline__ double norm_vel_f64(const gca_config& c, const Derive
   return ddiv_prepared(k, __dadd_rn(v, c.max_speed), k.dv_vel, k.rc_vel);
 }
 
-// the four entries of intruder i   PKG/SingleAircraftEnv.py:108-114 (raw: Simulators/SingleAircraftMCTSEnv.py:107-112)
-// `base` points at the first intruder entry of the env's observation row.
+// the four entries of an intruder   PKG/SingleAircraftEnv.py:108-114 (raw: Simulators/SingleAircraftMCTSEnv.py:107-112)
 template <bool FAITH>
 __device__ __forceinline__ void obs_intruder_entries(const StepArgs& a, const Intr<FAITH>& it, real_t<FAITH>& o0,
                                                      real_t<FAITH>& o1, real_t<FAITH>& o2, real_t<FAITH>& o3) {
@@ -493,29 +492,15 @@ __device__ __forceinline__ void obs_intruder_entries(const StepArgs& a, const In
   }
 }
 
+// the four entries of intruder i into its observation row; `base` points at the row's first intruder entry
 template <bool FAITH>
 __device__ __forceinline__ void write_obs_intruder(const StepArgs& a, real_t<FAITH>* base, int i,
                                                    const Intr<FAITH>& it) {
   using R = real_t<FAITH>;
   const gca_config& c = a.cfg;
-  const Derived& k = a.k;
   if (c.obs_kind == GCA_OBS_NONE || c.obs_kind == GCA_OBS_NEAREST || c.obs_kind == GCA_OBS_RAW6) return;   // (NEAREST: nearest_obs_kernel, RAW6: turn_obs_kernel)
   R o0, o1, o2, o3;
-  if (c.obs_kind == GCA_OBS_RAW) {
-    o0 = (R)it.px; o1 = (R)it.py; o2 = (R)it.vx; o3 = (R)it.vy;
-  } else {
-    bool wide = false;
-    if constexpr (FAITH) wide = it.is64;
-    if (wide) {
-      o0 = (R)ddiv_prepared(k, (double)it.px, k.dv_w, k.rc_w);
-      o1 = (R)ddiv_prepared(k, (double)it.py, k.dv_h, k.rc_h);
-    } else {
-      o0 = (R)div_prepared(k, (float)it.px, k.ob_w, k.inv_ob_w);
-      o1 = (R)div_prepared(k, (float)it.py, k.ob_h, k.inv_ob_h);
-    }
-    o2 = (R)norm_vel_f32(k, it.vx);
-    o3 = (R)norm_vel_f32(k, it.vy);
-  }
+  obs_intruder_entries<FAITH>(a, it, o0, o1, o2, o3);
   R* p = base + 4 * (size_t)i;
   if constexpr (FAITH) {
     reinterpret_cast<double2*>(p)[0] = make_double2(o0, o1);

@@ -49,11 +49,9 @@ __device__ __forceinline__ void copy_words(uint8_t* dst, const uint8_t* src, int
   for (int i = lane; i < nbytes / 4; i += 32) reinterpret_cast<uint32_t*>(dst)[i] = reinterpret_cast<const uint32_t*>(src)[i];
 }
 
-#ifndef GCA_HER_MINB
-#define GCA_HER_MINB 3                            // blocks per SM (80 registers): 7 % more transitions/s than 2, 4 and 6 spill
-#endif
+constexpr int kHerMinBlocks = 3;                  // blocks per SM (80 registers): 7 % more transitions/s than 2, 4 and 6 spill
 template <typename R>
-__global__ void __launch_bounds__(256, GCA_HER_MINB) her_sample_kernel(const HerArgs a) {
+__global__ void __launch_bounds__(256, kHerMinBlocks) her_sample_kernel(const HerArgs a) {
   const int lane = threadIdx.x & 31;
   const long long warps = (long long)gridDim.x * (blockDim.x >> 5);
   const size_t ro = (size_t)a.dim_o * sizeof(R), ru = (size_t)a.dim_u * sizeof(R), rg = (size_t)a.dim_g * sizeof(R);

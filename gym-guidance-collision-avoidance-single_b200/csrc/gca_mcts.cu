@@ -430,18 +430,14 @@ __global__ void __launch_bounds__(kPackThreads, 2) mcts_playout_packed_kernel(co
 // indices - the draws of intruder i are addressed by i), and every lane then runs its playout sequentially on a
 // private copy of the survivors (thread-local arrays: position, velocity and heading change per playout) - the same
 // operations in the same order per playout and intruder as the warp kernel, so the same bits.
-#ifndef GCA_LANE_THREADS
-#define GCA_LANE_THREADS 256
-#endif
-#ifndef GCA_LANE_MINB
-#define GCA_LANE_MINB 3
-#endif
-constexpr int kLaneThreads = GCA_LANE_THREADS;     // measured at 100 playouts per root: 256 threads (2 roots, 200 of 224 lanes), 3 CTAs per SM at 79
-                                                   // registers: 4.3e8 rollouts/s; 512 x 1 (112 registers) 3.6e8, 512 x 2 / 128 x 8 (64, spills) 3.8e8
+// measured at 100 playouts per root: 256 threads (2 roots, 200 of 224 lanes), 3 CTAs per SM at 79 registers: 4.3e8
+// rollouts/s; 512 x 1 (112 registers) 3.6e8, 512 x 2 / 128 x 8 (64, spills) 3.8e8
+constexpr int kLaneThreads = 256;
+constexpr int kLaneMinBlocks = 3;
 constexpr int kLaneMaxRoots = 8;
 constexpr int kLaneMaxNear = 80;              // thread-local arrays; larger models take the warp-per-playout kernel
 
-__global__ void __launch_bounds__(kLaneThreads, GCA_LANE_MINB) mcts_playout_rnd_lane_kernel(const MctsArgs a, const int R) {
+__global__ void __launch_bounds__(kLaneThreads, kLaneMinBlocks) mcts_playout_rnd_lane_kernel(const MctsArgs a, const int R) {
   extern __shared__ __align__(16) uint8_t mcts_sh[];
   const gca_mcts_config& c = a.c;
   const int F = c.simulate_frame, near = a.near;

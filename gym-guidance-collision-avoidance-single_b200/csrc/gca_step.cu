@@ -54,7 +54,10 @@ __device__ __forceinline__ unsigned long long gtime() {
 }
 __device__ unsigned long long g_cta[8192 * 2];   // per block of the streaming kernel: first instruction, last instruction
 extern "C" int gca_debug_cta(unsigned long long* host) { return (int)cudaMemcpyFromSymbol(host, g_cta, sizeof(g_cta)); }
-__device__ unsigned long long g_fin[2048 * 8];   // per tile: finish start, end, respawn iterations, resets
+// per tile: finish start, end, respawn records, resets, phase stamps.  Respawn records (PHILOX only; TAPE tiles leave the
+// slot alone): the records the spawn phase ran, capped at kTileRespawnCap, including records of envs that reset and were
+// skipped, excluding the respawns made in place (list full, or N > 128)
+__device__ unsigned long long g_fin[2048 * 8];
 extern "C" int gca_debug_fin(unsigned long long* host) { return (int)cudaMemcpyFromSymbol(host, g_fin, sizeof(g_fin)); }
 __device__ unsigned int g_lat[8 * 64];            // position-load latency of the streaming pass: [eighth of the walk][64-cycle bucket]
 extern "C" int gca_debug_lat(unsigned int* host, int clear) {
@@ -77,22 +80,51 @@ extern "C" int gca_debug_kstamps(unsigned long long* host, int reset) {
 #define GCA_KSTAMP_OUT(kid) do { } while (0)
 #endif
 
-#ifndef GCA_CHUNK_UNITS
-#define GCA_CHUNK_UNITS 4
-#endif
-#ifndef GCA_WARPS_B
-#define GCA_WARPS_B 4
-#endif
-#ifndef GCA_FAITH_MINB
-#define GCA_FAITH_MINB 1                          // blocks per SM the FAITHFUL streaming kernel is compiled for
-#endif
-constexpr int kChunkUnits = GCA_CHUNK_UNITS;      // 16-byte units (intruder pairs) per lane and work item
+constexpr int kChunkUnits = 4;                   // 16-byte units (intruder pairs) per lane and work item
 constexpr int kChunkIntr = 2 * kChunkUnits;       // 8 intruders
 constexpr int kTileRespawnCap = 128;              // respawn records per tile (32 envs) and step; beyond that the lane spawns in place
-constexpr int kWarpsB = GCA_WARPS_B;              // work items per block of the streaming pass
-// staging row of one lane: 8 intruders x 16 bytes of observation entries, plus 16 bytes so that the row stride is
-// an odd multiple of 16 (conflict-free 16-byte shared accesses across a quarter warp)
+constexpr int kWarpsB = 4;                        // work items per block of the streaming pass
+constexpr int kFaithMinBlocks = 1;                // blocks per SM the FAITHFUL streaming kernel is compiled for
+// staging row of one lane: 8 intruders x 16 bytes of observation entries (FAITHFUL: 32 bytes), plus 16 bytes so that
+// the row stride is an odd multiple of 16 (conflict-free 16-byte shared accesses across a quarter warp)
 constexpr uint32_t kObsRow = 16u * kChunkIntr + 16u;
+constexpr uint32_t kObsRow64 = 32u * kChunkIntr + 16u;
+static_assert(32 % kChunkIntr == 0, "the event bits of a work item must not straddle a word, and the FAST write-out "
+                                    "stores 32 / kChunkIntr whole env rows per instruction");
+static_assert(32 * kChunkIntr == 16 * 16, "the FAITHFUL write-out stores one env's work item with 16 lanes x 16 bytes");
+static_assert(kWarpsB * 32 * kObsRow64 <= 0xc000, "the FAITHFUL staging buffer must fit in static shared memory");
+
+// spawn() of intruder i of env `env` (slot: i for reset_intruder() :229-238, GCA_SLOT_RESET | i for reset() :80-88) and
+// its stores: position into `plane`, velocity, observation entries into the env's row `obase` (obs_intruder_base).
+// Returns whether the position is f64 (Q3).
+template <bool FAITH, bool TAPE>
+__device__ __forceinline__ bool spawn_store(const StepArgs& a, Draws<TAPE>& d, uint32_t slot, size_t env, int i, int plane,
+                                            float ox, float oy, real_t<FAITH>* obase) {
+  const DevState& s = a.s;
+  Intr<FAITH> it;
+  spawn<FAITH, TAPE>(d, a.cfg, a.k, slot, ox, oy, it, ihs_slot(s, env, i));
+  store_ipos<FAITH>(s, plane, env, i, it);
+  store_ivel(s, env, i, it.vx, it.vy);
+  write_obs_intruder<FAITH>(a, obase, i, it);
+  return it.is64;
+}
+
+// reset()'s spawns of intruders 32 r .. 32 r + 31 of env `env`, one per lane, then the word's flags: conflict False,
+// FAITHFUL the f64 bits of the new positions.  Executed by the whole warp; PHILOX only (the draws are independent).
+template <bool FAITH>
+__device__ __forceinline__ void spawn_reset_word(const StepArgs& a, Draws<false>& d, size_t env, int r, int lane, int plane,
+                                                 const float2& own) {
+  const DevState& s = a.s;
+  const int i = r * 32 + lane;
+  bool wide = false;
+  if (i < s.N)
+    wide = spawn_store<FAITH, false>(a, d, GCA_SLOT_RESET | (uint32_t)i, env, i, plane, own.x, own.y, obs_intruder_base<FAITH>(a, env));
+  const uint32_t dw = __ballot_sync(FULL, wide);
+  if (lane == 0) {
+    s.cflag[flag_index(s, env, r)] = 0u;
+    if constexpr (FAITH) s.dflag[flag_index(s, env, r)] = dw;
+  }
+}
 
 // reset(): PKG/SingleAircraftEnv.py:66-98 for env `env`, executed by the whole warp; positions go to `plane`.
 // PHILOX: lanes = intruders.  TAPE: lane `owner` replays the reference's sequential draw order.
@@ -101,8 +133,6 @@ __device__ __forceinline__ void reset_env_warp(const StepArgs& a, size_t env, in
                                                Draws<TAPE>& d, double2& goal, const float ox, const float oy) {
   const DevState& s = a.s;
   const gca_config& c = a.cfg;
-  const Derived& k = a.k;
-  real_t<FAITH>* obase = obs_intruder_base<FAITH>(a, env);
   // (ox, oy): the ownship the new intruders keep their distance from - (50, 50) :72-76, or the random start
   if constexpr (TAPE) {
     if (lane == owner) {
@@ -110,12 +140,8 @@ __device__ __forceinline__ void reset_env_warp(const StepArgs& a, size_t env, in
         uint32_t dw = 0;
         for (int j = 0; j < 32 && r * 32 + j < s.N; ++j) {
           const int i = r * 32 + j;
-          Intr<FAITH> it;
-          spawn<FAITH, TAPE>(d, c, k, GCA_SLOT_RESET | (uint32_t)i, ox, oy, it, ihs_slot(s, env, i));
-          store_ipos<FAITH>(s, plane, env, i, it);
-          store_ivel(s, env, i, it.vx, it.vy);
-          dw |= (it.is64 ? 1u : 0u) << j;
-          write_obs_intruder<FAITH>(a, obase, i, it);
+          const bool is64 = spawn_store<FAITH, TAPE>(a, d, GCA_SLOT_RESET | (uint32_t)i, env, i, plane, ox, oy, obs_intruder_base<FAITH>(a, env));
+          dw |= (is64 ? 1u : 0u) << j;
         }
         s.cflag[flag_index(s, env, r)] = 0u;
         if constexpr (FAITH) s.dflag[flag_index(s, env, r)] = dw;
@@ -123,26 +149,52 @@ __device__ __forceinline__ void reset_env_warp(const StepArgs& a, size_t env, in
       draw_goal(d, c, goal.x, goal.y);   // Goal(random_pos()) :93
     }
   } else {
-    for (int r = 0; r < s.W; ++r) {
-      const int i = r * 32 + lane;
-      const bool valid = i < s.N;
-      Intr<FAITH> it;
-      bool wide = false;
-      if (valid) {
-        spawn<FAITH, TAPE>(d, c, k, GCA_SLOT_RESET | (uint32_t)i, ox, oy, it, ihs_slot(s, env, i));
-        store_ipos<FAITH>(s, plane, env, i, it);
-        store_ivel(s, env, i, it.vx, it.vy);
-        write_obs_intruder<FAITH>(a, obase, i, it);
-        wide = it.is64;
-      }
-      const uint32_t dw = __ballot_sync(FULL, wide);
-      if (lane == 0) {
-        s.cflag[flag_index(s, env, r)] = 0u;
-        if constexpr (FAITH) s.dflag[flag_index(s, env, r)] = dw;
-      }
-    }
+    const float2 own = make_float2(ox, oy);
+    for (int r = 0; r < s.W; ++r) spawn_reset_word<FAITH>(a, d, env, r, lane, plane, own);
     if (lane == owner) draw_goal(d, c, goal.x, goal.y);
   }
+}
+
+// reset() of every env of the warp's tile whose lane has `resets` set, one env at a time (the tape is sequential): the
+// ownship's draws first, then the intruders' and the goal's (reset_env_warp), then lane e's draws continue behind them.
+// On return a resetting lane holds its env's new pos / hs / vel / goal.  `nxt`: the plane the env's positions go to.
+template <bool FAITH, bool TAPE>
+__device__ __forceinline__ void reset_envs_warp(const StepArgs& a, size_t env0, int lane, bool resets, int nxt, Draws<TAPE>& d,
+                                                float2& pos, double2& hs, double2& vel, double2& goal) {
+  uint32_t rmask = __ballot_sync(FULL, resets);
+  while (rmask) {
+    const int e = __ffs(rmask) - 1;
+    rmask &= rmask - 1;
+    __syncwarp();                                                 // lane e's stores above come first
+    Draws<TAPE> de = d;
+    if constexpr (!TAPE) {
+      de.env = __shfl_sync(FULL, d.env, e);
+      de.tick = __shfl_sync(FULL, d.tick, e);
+    }
+    const int plane = __shfl_sync(FULL, nxt, e);
+    if (lane == e) reset_ownship<TAPE>(a.cfg, de, pos, hs, vel);  // (its draws come first on the tape)
+    const float rx = __shfl_sync(FULL, pos.x, e), ry = __shfl_sync(FULL, pos.y, e);
+    reset_env_warp<FAITH, TAPE>(a, env0 + e, plane, lane, e, de, goal, rx, ry);
+    if constexpr (TAPE) {
+      if (lane == e) d = de;
+    }
+  }
+}
+
+// the ownship side of reset() for env `me`: its state, no_conflict and ep_steps zeroed, the reset observation's
+// ownship / goal entries (f32 velocity, :76)
+template <bool FAITH>
+__device__ __forceinline__ void store_own_reset(const StepArgs& a, size_t me, float2 pos, double2 hs, double2 vel, double2 goal,
+                                                int4& cnt) {
+  const DevState& s = a.s;
+  s.own_pos[me] = pos;
+  s.own_hs[me] = hs;
+  s.own_vel[me] = vel;
+  s.own_vel_f32[me] = 1;
+  s.goal[me] = goal;
+  cnt.x = 0;
+  cnt.y = 0;
+  write_obs_own<FAITH>(a, me, pos.x, pos.y, vel.x, vel.y, true, hs.x, hs.y, goal.x, goal.y);
 }
 
 // ------------------------------------------------------------------------------ 1. ownship
@@ -279,7 +331,7 @@ __device__ __forceinline__ void finish_tile(const StepArgs& a, const int tile, c
   const size_t me = has_env ? env0 + lane : env0;
 #ifdef GCA_PHASE_TIMING
   const unsigned long long fin_t0 = gtime();
-  int fin_respawns = 0, fin_resets = 0;
+  int fin_resets = 0;
 #endif
 
   float2 pos = make_float2(0.f, 0.f);
@@ -349,12 +401,28 @@ __device__ __forceinline__ void finish_tile(const StepArgs& a, const int tile, c
   };
   // reset_intruder() for intruder i of this lane's env   :153-154, :229-238
   auto respawn_own = [&](int i, uint32_t& set64) {
-    Intr<FAITH> it;
-    spawn<FAITH, TAPE>(d, c, k, (uint32_t)i, pos.x, pos.y, it, ihs_slot(s, me, i));
-    store_ipos<FAITH>(s, nxt, me, i, it);
-    store_ivel(s, me, i, it.vx, it.vy);
-    set64 |= (it.is64 ? 1u : 0u) << (i & 31);
-    write_obs_intruder<FAITH>(a, obase, i, it);
+    set64 |= (spawn_store<FAITH, TAPE>(a, d, (uint32_t)i, me, i, nxt, pos.x, pos.y, obase) ? 1u : 0u) << (i & 31);
+  };
+  // the loop's events in word w of this lane's env (conf, gone: the visited intruders; cf: the conflict word before the
+  // step).  in_place: respawn here, in index order (TAPE: the reference's draw order); else the spawn phase does it.
+  auto replay_word = [&](int w, uint32_t conf, uint32_t gone, uint32_t cf, bool in_place) {
+    const size_t fi = flag_index(s, me, w);
+    newconf += __popc(conf & ~cf);                        // False -> True transitions :161-163 (old object's flag, Q7)
+    conf_any |= conf != 0u;
+    const uint32_t ncf = (cf | conf) & ~gone;             // the flag never clears (Q8); a replaced intruder starts False
+    if (ncf != cf) s.cflag[fi] = ncf;
+    uint32_t set64 = 0;
+    if (in_place) {
+      uint32_t rest = gone;
+      while (rest) {
+        const int j = __ffs(rest) - 1;
+        rest &= rest - 1;
+        respawn_own(w * 32 + j, set64);
+      }
+    }
+    if constexpr (FAITH) {
+      if (gone) s.dflag[fi] = (s.dflag[fi] & ~gone) | set64;
+    }
   };
 
   // self.dist_nearest_intruder (Simulators/SingleAircraftDiscrete3HEREnv.py:185,191): min over the intruders the loop
@@ -391,26 +459,9 @@ __device__ __forceinline__ void finish_tile(const StepArgs& a, const int tile, c
 #pragma unroll
       for (int w = 0; w < kWordsAhead; ++w) {
         const uint32_t vis = visited_mask(w);
-        const uint32_t conf = wc[w] & vis, gone = wg[w] & vis, cf = wf[w];
+        const uint32_t conf = wc[w] & vis, gone = wg[w] & vis;
         wg[w] = gone;
-        if ((conf | gone) == 0u) continue;
-        const size_t fi = flag_index(s, me, w);
-        newconf += __popc(conf & ~cf);                    // False -> True transitions :161-163 (old object's flag, Q7)
-        conf_any |= conf != 0u;
-        const uint32_t ncf = (cf | conf) & ~gone;         // the flag never clears (Q8); a replaced intruder starts False
-        if (ncf != cf) s.cflag[fi] = ncf;
-        uint32_t set64 = 0;
-        if (!compact) {                                   // TAPE: this lane replays its env's draws in index order
-          uint32_t rest = gone;
-          while (rest) {
-            const int j = __ffs(rest) - 1;
-            rest &= rest - 1;
-            respawn_own(w * 32 + j, set64);
-          }
-        }
-        if constexpr (FAITH) {
-          if (gone) s.dflag[fi] = (s.dflag[fi] & ~gone) | set64;
-        }
+        if (conf | gone) replay_word(w, conf, gone, wf[w], !compact);
       }
     } else {
       for (int w = 0; w < s.W; ++w) {                     // N > 128: word by word
@@ -422,21 +473,7 @@ __device__ __forceinline__ void finish_tile(const StepArgs& a, const int tile, c
           if (gone_all) s.ev_gone[fi] = 0u;
         }
         const uint32_t conf = conf_all & vis, gone = gone_all & vis;
-        if ((conf | gone) == 0u) continue;
-        const uint32_t cf = s.cflag[fi];
-        newconf += __popc(conf & ~cf);
-        conf_any |= conf != 0u;
-        const uint32_t ncf = (cf | conf) & ~gone;
-        if (ncf != cf) s.cflag[fi] = ncf;
-        uint32_t rest = gone, set64 = 0;
-        while (rest) {
-          const int j = __ffs(rest) - 1;
-          rest &= rest - 1;
-          respawn_own(w * 32 + j, set64);
-        }
-        if constexpr (FAITH) {
-          if (gone) s.dflag[fi] = (s.dflag[fi] & ~gone) | set64;
-        }
+        if (conf | gone) replay_word(w, conf, gone, s.cflag[fi], true);
       }
     }
   }
@@ -571,18 +608,7 @@ __device__ __forceinline__ void finish_tile(const StepArgs& a, const int tile, c
   const bool resets = a.auto_reset && has_env && done;
   int reset_slot = -1;
   if constexpr (TAPE) {
-    uint32_t dmask = __ballot_sync(FULL, resets);
-    while (dmask) {                                                 // the tape is sequential: one env at a time
-      const int e = __ffs(dmask) - 1;
-      dmask &= dmask - 1;
-      __syncwarp();                                                 // lane e's stores above come first
-      Draws<TAPE> de = d;
-      const int plane = __shfl_sync(FULL, nxt, e);
-      if (lane == e) reset_ownship<TAPE>(c, de, pos, hs, vel);       // (its draws come first on the tape)
-      const float rx = __shfl_sync(FULL, pos.x, e), ry = __shfl_sync(FULL, pos.y, e);
-      reset_env_warp<FAITH, TAPE>(a, env0 + e, plane, lane, e, de, goal, rx, ry);
-      if (lane == e) d = de;
-    }
+    reset_envs_warp<FAITH, TAPE>(a, env0, lane, resets, nxt, d, pos, hs, vel, goal);
   } else {
     // PHILOX: the 80 spawns of each finished env are independent of everything else; they are queued for
     // reset_spawn_kernel (one warp per 32 of them, all finished envs of the batch at once) instead of
@@ -610,15 +636,8 @@ __device__ __forceinline__ void finish_tile(const StepArgs& a, const int tile, c
         bs->tick[reset_slot] = cnt.z;
       }
     }
-    s.own_pos[me] = pos;
-    s.own_hs[me] = hs;
-    s.own_vel[me] = vel;
-    s.own_vel_f32[me] = 1;
-    s.goal[me] = goal;
-    cnt.x = 0;
-    cnt.y = 0;
     cnt.w += 1;
-    write_obs_own<FAITH>(a, me, pos.x, pos.y, vel.x, vel.y, true, hs.x, hs.y, goal.x, goal.y);
+    store_own_reset<FAITH>(a, me, pos, hs, vel, goal, cnt);
   }
   if (has_env) {
     cnt.z += 1;                                                     // Philox tick; also flips the current position plane
@@ -627,7 +646,7 @@ __device__ __forceinline__ void finish_tile(const StepArgs& a, const int tile, c
   }
 #ifdef GCA_PHASE_TIMING
   if (lane == 0 && tile < 2048) {
-    g_fin[tile * 8 + 0] = fin_t0; g_fin[tile * 8 + 1] = gtime(); g_fin[tile * 8 + 2] = fin_respawns; g_fin[tile * 8 + 3] = fin_resets;
+    g_fin[tile * 8 + 0] = fin_t0; g_fin[tile * 8 + 1] = gtime(); g_fin[tile * 8 + 3] = fin_resets;
     g_fin[tile * 8 + 4] = fin_t1; g_fin[tile * 8 + 5] = fin_t2; g_fin[tile * 8 + 6] = fin_t3;
   }
 #endif
@@ -657,42 +676,28 @@ __device__ __forceinline__ void spawn_phase(const StepArgs& a, const int tile, c
       const float2 own = ws->pos[e];
       d.env = a.env_id0 + (uint32_t)env;
       d.tick = (uint32_t)tick;
-      Intr<FAITH> it;
-      spawn<FAITH, false>(d, a.cfg, a.k, (uint32_t)i, own.x, own.y, it, ihs_slot(s, env, i));
-      store_ipos<FAITH>(s, (tick & 1) ^ 1, env, i, it);     // the plane this step wrote
-      store_ivel(s, env, i, it.vx, it.vy);
-      write_obs_intruder<FAITH>(a, obs_intruder_base<FAITH>(a, env), i, it);
+      const bool is64 = spawn_store<FAITH, false>(a, d, (uint32_t)i, env, i, (tick & 1) ^ 1, own.x, own.y,   // (the plane this step wrote)
+                                                  obs_intruder_base<FAITH>(a, env));
       if constexpr (FAITH) {
-        if (it.is64) atomicOr(&s.dflag[flag_index(s, env, i >> 5)], 1u << (i & 31));
+        if (is64) atomicOr(&s.dflag[flag_index(s, env, i >> 5)], 1u << (i & 31));
       }
     }
   }
 #ifdef GCA_PHASE_TIMING
-  if (lane == 0 && tile < 2048 && tile < s.T) g_fin[tile * 8 + 7] = gtime();
+  if (lane == 0 && tile < 2048 && tile < s.T) {
+    g_fin[tile * 8 + 2] = ws->n_jobs;
+    g_fin[tile * 8 + 7] = gtime();
+  }
 #endif
   __syncthreads();                                          // every warp's resets are queued, their scalar state stored
   const int rounds = s.W, total = bs->count * rounds;
   for (int job = wib; job < total; job += 4) {
     const size_t env = (size_t)bs->env[job / rounds];
-    const int r = job % rounds, i = r * 32 + lane;
+    const int r = job % rounds;
     const int tick = bs->tick[job / rounds];                // the tick of the step that finished the env
     d.env = a.env_id0 + (uint32_t)env;
     d.tick = (uint32_t)tick;
-    bool wide = false;
-    if (i < s.N) {
-      Intr<FAITH> it;
-      const float2 own = bs->pos[job / rounds];             // (50, 50) :72-76, or the random start finish_tile drew
-      spawn<FAITH, false>(d, a.cfg, a.k, GCA_SLOT_RESET | (uint32_t)i, own.x, own.y, it, ihs_slot(s, env, i));
-      store_ipos<FAITH>(s, (tick & 1) ^ 1, env, i, it);      // the plane this step wrote = the env's next current plane
-      store_ivel(s, env, i, it.vx, it.vy);
-      write_obs_intruder<FAITH>(a, obs_intruder_base<FAITH>(a, env), i, it);
-      wide = it.is64;
-    }
-    const uint32_t dw = __ballot_sync(FULL, wide);
-    if (lane == 0) {
-      s.cflag[flag_index(s, env, r)] = 0u;
-      if constexpr (FAITH) s.dflag[flag_index(s, env, r)] = dw;
-    }
+    spawn_reset_word<FAITH>(a, d, env, r, lane, (tick & 1) ^ 1, bs->pos[job / rounds]);   // (the plane this step wrote)
   }
 }
 
@@ -746,7 +751,7 @@ __global__ void __launch_bounds__(128, MINB) step_n0_kernel(const __grid_constan
 // DRIFT: every advance adds Config.position_sigma to the velocity (the random-intruder env); generic layout only, so the
 // instruction streams of the other instantiations are what they were without it.
 template <bool FAITH, int OM, bool DRIFT = false>
-__global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : 1) step_intruders_kernel(const __grid_constant__ StepArgs a) {
+__global__ void __launch_bounds__(kWarpsB * 32, FAITH ? kFaithMinBlocks : 1) step_intruders_kernel(const __grid_constant__ StepArgs a) {
   static_assert(!(DRIFT && OM), "a handle with a position drift takes the generic observation path");
   pdl_wait();
   GCA_KSTAMP_IN(1);
@@ -756,7 +761,6 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : 1) step
   using R = real_t<FAITH>;
   static_assert(!(FAITH && OM), "the specialised observation path is FAST only");
   // observation staging: FAST specialised layouts 8 x 16 bytes per lane, FAITHFUL 8 x 32 bytes per lane (+ 16: odd stride)
-  constexpr uint32_t kObsRow64 = 32u * kChunkIntr + 16u;
   constexpr uint32_t kWarpSmem = OM ? 32 * kObsRow : (FAITH ? 32 * kObsRow64 : 16);
   constexpr uint32_t kStageBytes = kWarpsB * kWarpSmem;
   __shared__ __align__(16) uint8_t stage_smem[kStageBytes];
@@ -1068,7 +1072,6 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? GCA_FAITH_MINB : 1) step
 template <bool FAITH, bool TAPE>
 __global__ void __launch_bounds__(128) reset_kernel(const StepArgs a) {
   const DevState& s = a.s;
-  const gca_config& c = a.cfg;
   const int lane = threadIdx.x & 31;
   const long long tile = (long long)blockIdx.x * 4 + (threadIdx.x >> 5);
   if (tile >= s.T) return;
@@ -1080,39 +1083,16 @@ __global__ void __launch_bounds__(128) reset_kernel(const StepArgs a) {
   if (has_env) cnt = s.counters[me];
   Draws<TAPE> d = make_draws<TAPE>(a, me, (uint32_t)cnt.z);
   const int nxt = (cnt.z & 1) ^ 1;                       // a reset is a tick too: it writes the other plane
-  uint32_t rmask = __ballot_sync(FULL, selected);
-  while (rmask) {
-    const int e = __ffs(rmask) - 1;
-    rmask &= rmask - 1;
-    __syncwarp();
-    Draws<TAPE> de = d;
-    if constexpr (!TAPE) {
-      de.env = __shfl_sync(FULL, d.env, e);
-      de.tick = __shfl_sync(FULL, d.tick, e);
-    }
-    const int plane = __shfl_sync(FULL, nxt, e);
-    double2 goal = make_double2(0., 0.);
-    float2 pos = make_float2(0.f, 0.f);
-    double2 hs = make_double2(0., 0.), vel = make_double2(0., 0.);
-    if (lane == e) reset_ownship<TAPE>(c, de, pos, hs, vel);         // (its draws come first on the tape)
-    const float rx = __shfl_sync(FULL, pos.x, e), ry = __shfl_sync(FULL, pos.y, e);
-    reset_env_warp<FAITH, TAPE>(a, env0 + e, plane, lane, e, de, goal, rx, ry);
-    if (lane == e) {
-      if constexpr (TAPE) d = de;
-      s.own_pos[me] = pos;
-      s.own_hs[me] = hs;
-      s.own_vel[me] = vel;
-      s.own_vel_f32[me] = 1;
-      s.goal[me] = goal;
-      cnt.x = 0;
-      cnt.y = 0;
-      cnt.z += 1;
-      s.counters[me] = cnt;
-      if constexpr (TAPE) a.cursor[me] = d.cur;
-      if (a.done) a.done[me] = 0;
-      if (a.info) a.info[me] = 0;
-      write_obs_own<FAITH>(a, me, pos.x, pos.y, vel.x, vel.y, true, hs.x, hs.y, goal.x, goal.y);
-    }
+  float2 pos = make_float2(0.f, 0.f);
+  double2 hs = make_double2(0., 0.), vel = make_double2(0., 0.), goal = make_double2(0., 0.);
+  reset_envs_warp<FAITH, TAPE>(a, env0, lane, selected, nxt, d, pos, hs, vel, goal);
+  if (selected) {
+    store_own_reset<FAITH>(a, me, pos, hs, vel, goal, cnt);
+    cnt.z += 1;
+    s.counters[me] = cnt;
+    if constexpr (TAPE) a.cursor[me] = d.cur;
+    if (a.done) a.done[me] = 0;
+    if (a.info) a.info[me] = 0;
   }
 }
 

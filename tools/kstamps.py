@@ -92,6 +92,7 @@ print("finish_tile per tile (us): mean %.2f p50 %.2f p90 %.2f p99 %.2f max %.2f"
 print("finish phases (us, mean): loads %.2f  replay %.2f  reward+stores %.2f  reset+counters %.2f  spawn phase (i) %.2f" % (
     ((f[:, 4] - f[:, 0]) / 1e3).mean(), ((f[:, 5] - f[:, 4]) / 1e3).mean(), ((f[:, 6] - f[:, 5]) / 1e3).mean(),
     ((f[:, 1] - f[:, 6]) / 1e3).mean(), ((f[:, 7] - f[:, 1]) / 1e3).mean()))
+print("per tile (mean): respawn records %.2f, resets %.2f" % (f[:, 2].mean(), f[:, 3].mean()))
 t0 = f[:, 0].min()
 print("relative to the first finish warp: finish_tile starts p50 %.2f max %.2f; ends max %.2f; spawn (i) ends max %.2f" % (
     (np.median(f[:, 0]) - t0) / 1e3, (f[:, 0].max() - t0) / 1e3, (f[:, 1].max() - t0) / 1e3, (f[:, 7].max() - t0) / 1e3))
