@@ -700,6 +700,15 @@ int gca_raster(gca_env* e, const uint8_t* sprites, uint8_t* frames, int64_t env_
     return fail(GCA_ERR_STATE, "the rasteriser needs an integer window with width % 16 == 0 and height % 4 == 0");
   if (n_planes < 1 || slot < 0 || slot >= n_planes) return fail(GCA_ERR_INVALID, "bad plane selection");
   if (plane_stride % 4 || env_stride % 4) return fail(GCA_ERR_INVALID, "strides must be multiples of 4 bytes");
+  // the kernel reads sprites and writes frames 4 bytes at a time: with the stride rule above, 4-byte aligned
+  // pointers make every such access aligned
+  if (reinterpret_cast<uintptr_t>(frames) % 4) return fail(GCA_ERR_INVALID, "frames must be 4-byte aligned");
+  if (reinterpret_cast<uintptr_t>(sprites) % 4) return fail(GCA_ERR_INVALID, "sprites must be 4-byte aligned");
+  if (raster_smem_bytes(W / 4, H / 4) > kRasterSmemMax || W / 4 > 32767 || H / 4 > 32767)
+    return fail(GCA_ERR_STATE, "the rasteriser keeps the whole " + std::to_string(W / 4) + "x" + std::to_string(H / 4) +
+                                   " output plane of the " + std::to_string(W) + "x" + std::to_string(H) +
+                                   " canvas in shared memory: " + std::to_string(raster_smem_bytes(W / 4, H / 4)) +
+                                   " bytes, more than the " + std::to_string(kRasterSmemMax) + " a block may use");
   GCA_CUDA(cudaSetDevice(e->device));
   GCA_CUDA(launch_raster(e->s, e->mode == GCA_MODE_FAITHFUL, W, H, sprites, frames, (long long)env_stride,
                          (long long)plane_stride, n_planes, slot, clear_mask, (cudaStream_t)stream));

@@ -46,6 +46,8 @@ cudaError_t launch_stats_update(const uint8_t* done, const uint8_t* info, long l
 cudaError_t launch_her_sample(const gca_her_episodes* ep, long long E, int T, int dim_o, int dim_u, int dim_g, int is_f64,
                               long long batch, double future_p, double radius, int kind, const gca_her_draws* dr,
                               uint64_t seed, uint32_t call, const gca_her_transitions* out, cudaStream_t st);
+constexpr size_t kRasterSmemMax = 227 * 1024;   // dynamic shared memory one block may use
+size_t raster_smem_bytes(int ow, int oh);        // what raster_kernel needs for an ow x oh output plane
 cudaError_t launch_raster(const DevState& s, bool faithful, int W, int H, const uint8_t* sprites, uint8_t* frames,
                           long long env_stride, long long plane_stride, int n_planes, int slot,
                           const uint8_t* clear_mask, cudaStream_t st);

@@ -497,12 +497,12 @@ cudaError_t launch_raster(const DevState& s, bool faithful, int W, int H, const 
   a.bulk_ok = ((a.ow * a.oh) % 16 == 0 && env_stride % 16 == 0 && plane_stride % 16 == 0 &&
                reinterpret_cast<uintptr_t>(frames) % 16 == 0) ? 1 : 0;
   const size_t smem = raster_smem_bytes(a.ow, a.oh);
-  if (smem > 227 * 1024 || a.ow > 32767 || a.oh > 32767) return cudaErrorInvalidValue;
+  if (smem > kRasterSmemMax || a.ow > 32767 || a.oh > 32767) return cudaErrorInvalidValue;
   cudaError_t e = cudaFuncSetAttribute(raster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   int dev = 0, sms = 148;
   if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  const int per_sm = smem * 2 + 2048 <= 227 * 1024 ? 2 : 1;
+  const int per_sm = smem * 2 + 2048 <= kRasterSmemMax ? 2 : 1;
   const unsigned grid = (unsigned)min((long long)s.B, (long long)sms * per_sm);
   raster_kernel<<<grid, kRasterThreads, smem, st>>>(a);
   return cudaGetLastError();

@@ -420,10 +420,16 @@ int gca_mcts_search(const gca_mcts_config* cfg, int n_intruders, const double* r
  * against the few sprites whose bounding box touches its cell.  DESIGN.md section 4.5 is the spec
  * (the GL half of the reference cannot run without a display, so the restatement is the spec).
  *
- * sprites: device uint8 [3][32][32][4] = (ownship, goal, intruder) x rows top->bottom x RGBA.
- * frames : device uint8; env b writes (H/4)*(W/4) bytes at frames + b*env_stride + slot*plane_stride.
+ * sprites: device uint8 [3][32][32][4] = (ownship, goal, intruder) x rows top->bottom x RGBA, 4-byte aligned.
+ * frames : device uint8, 4-byte aligned; env b writes (H/4)*(W/4) bytes at frames + b*env_stride + slot*plane_stride.
+ *          env_stride and plane_stride are multiples of 4.  When frames, both strides and the plane size are
+ *          multiples of 16 a plane leaves with one bulk copy, otherwise with 4-byte stores (same bytes).
  * clear_mask (nullable, device uint8 [B]): for a non-zero entry the other n_planes-1 planes of that env
- * are zero-filled first - VecFrameStack's reset of a finished env (vec_frame_stack.py:19-23, Q21). */
+ * are zero-filled first - VecFrameStack's reset of a finished env (vec_frame_stack.py:19-23, Q21).
+ * GCA_ERR_INVALID for an unaligned pointer or stride; GCA_ERR_STATE for a window whose width is not a multiple
+ * of 16 or height not a multiple of 4, and for one whose output plane, with about 70 KB of textures and tables,
+ * does not fit in the 227 KB of shared memory a block may use (1600x1504 fits, 1600x1600 does not).  Neither
+ * launches a kernel. */
 #define GCA_RASTER_MAX_INTRUDERS 126
 int gca_raster(gca_env* env, const uint8_t* sprites, uint8_t* frames, int64_t env_stride, int64_t plane_stride,
                int n_planes, int slot, const uint8_t* clear_mask, void* stream);

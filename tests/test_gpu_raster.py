@@ -48,13 +48,24 @@ def test_frames_match_independent_renderer_gpu():
     print("pixels differing from the independent renderer:", differ)
 
 
+def _sm_count():
+    import torch
+    return torch.cuda.get_device_properties(0).multi_processor_count
+
+
+# B = 1000 (> 3 x 2 x 148, not a multiple of the persistent grid of either 1 or 2 CTAs per SM): every CTA rasterises
+# several envs, so the crowded envs below land on a CTA's second and third iteration too
 @pytest.mark.parametrize("n,B,mode,which", [(80, 24, "fast", "reference"), (80, 8, "faithful", "reference"), (0, 4, "fast", "reference"),
                                             (126, 6, "fast", "reference"), (5, 40, "fast", "reference"), (80, 24, "fast", "lookalike"),
-                                            (33, 16, "faithful", "lookalike")])
+                                            (33, 16, "faithful", "lookalike"), (80, 1000, "fast", "reference"),
+                                            (80, 1000, "faithful", "lookalike"), (126, 1000, "fast", "reference"),
+                                            (0, 1000, "fast", "reference")])
 def test_frames_equal_cpu_restatement(n, B, mode, which):
     import torch
     from gca_b200.stack import ImageBatch
     from oracle import oracle as orc
+    if B >= 1000:
+        assert B >= 3 * 2 * _sm_count() and B % _sm_count() != 0
     sp = _sprite_set(which)
     env = ImageBatch(B, _cfg(), n_intruders=n, mode=mode, seed=11, sprites=sp)
     ref = orc.OracleEnv(variants.make_config("SingleAircraftStackEnv", _cfg()), B, n, draws=1, trig=orc.TRIG_SHARED,
@@ -82,10 +93,12 @@ def test_frames_equal_cpu_restatement(n, B, mode, which):
     env.close()
 
 
-def test_frame_stack_ring_equals_vec_frame_stack():
+def check_frame_stack_ring(B):
+    """The k-plane ring against VecFrameStack's roll / zero-on-done semantics over 9 steps; returns how many envs past
+    every CTA's first one (rows >= 2 x SMs) were zero-filled while all their older planes held a picture."""
     import torch
     from gca_b200.stack import ImageBatch
-    B, k = 12, 4
+    k = 4
     cfg = _cfg()
     env = ImageBatch(B, cfg, n_intruders=20, frame_stack=k, seed=3, sprites=_sprite_set("reference"))
     first = env.reset().cpu().numpy()
@@ -93,21 +106,34 @@ def test_frame_stack_ring_equals_vec_frame_stack():
     stacked[..., -1:] = first
     assert np.array_equal(env.stacked().cpu().numpy(), stacked)
     rng = np.random.RandomState(0)
-    st = env.batch.get_state()
-    st["goal"][:4] = st["own_pos"][:4] + 25.0               # a few envs reach the goal soon -> done -> stack reset
-    env.batch.set_state(st)
-    seen_done = 0
+    later = 2 * _sm_count()                                  # rows past every CTA's first env, for 1 or 2 CTAs per SM
+    cleared_late = seen_done = 0
     for t in range(9):
+        # the goal on the ownship: a residue class of rows, spread over the batch, finishes at this step -> stack reset
+        # (unless an intruder inside the separation radius outranks the goal)
+        st = env.batch.get_state()
+        plant = np.arange(B) % 5 == t % 5
+        st["goal"][plant] = st["own_pos"][plant]
+        env.batch.set_state({"goal": st["goal"]})
         a = torch.as_tensor(rng.randint(0, 9, B).astype(np.int32), device="cuda")
         frame, rew, done, info = env.step(a)
         d = done.cpu().numpy().astype(bool)
         stacked = np.roll(stacked, shift=-1, axis=-1)        # vec_frame_stack.py:17-24
+        # envs past every CTA's first one whose k - 1 older planes all hold a picture that the zero-fill must erase
+        older = stacked[d & (np.arange(B) >= later)][..., :-1]
+        cleared_late += int((older != 0).any(axis=(1, 2)).all(1).sum())
         stacked[d] = 0
         stacked[..., -1:] = frame.cpu().numpy()
         assert np.array_equal(env.stacked().cpu().numpy(), stacked), t
+        assert d[plant].any(), t
         seen_done += int(d.sum())
     assert seen_done > 0
     env.close()
+    return cleared_late
+
+
+def test_frame_stack_ring_equals_vec_frame_stack():
+    check_frame_stack_ring(12)
 
 
 def test_stack_env_facade_rules():

@@ -68,6 +68,42 @@ def test_render_geometry():
     assert np.abs(iq.astype(int) - np.rot90(np.rint(sp[2, :, :, :3] * (sp[2, :, :, 3:4] / 255.0) + 255 * (1 - sp[2, :, :, 3:4] / 255.0)), -1)).max() <= 1
 
 
+@pytest.mark.parametrize("W,H,W2,H2", [(800, 800, 800, 804), (800, 800, 816, 800), (800, 800, 1600, 1504),
+                                       (64, 64, 640, 480)])
+def test_render_geometry_carries_to_other_canvases(W, H, W2, H2):
+    """Only the 800 x 800 canvas is pinned against cv2 and the independent renderer.  A scene drawn on a W2 x H2 canvas
+    with every y raised by H2 - H and x unchanged must give, in its first H/4 rows and W/4 columns, the frame of the
+    W x H canvas: the top edge, the left edge and every sample stay where they were.  Positions are multiples of 1/256,
+    so y + (H2 - H) and every sample's offset from a centre are exact in f32."""
+    from gym_guidance_collision_avoidance_single.envs.config import Config
+    B, N = 6, 40
+    rng = np.random.RandomState(W2 * 7 + H2)
+    q = lambda x: np.round(np.asarray(x) * 256.0) / 256.0
+    envs = []
+    for w, h in ((W, H), (W2, H2)):
+        cls = type("Cfg%dx%d" % (w, h), (Config,), dict(window_width=w, window_height=h))
+        envs.append(orc.OracleEnv(variants.make_config("SingleAircraftStackEnv", cls), B, N, draws=1,
+                                  trig=orc.TRIG_SHARED, seed=4))
+    st = envs[0].state
+    # crowded, and across all four edges of the smaller canvas
+    st["own_pos"][:] = q(rng.uniform(-20, [W + 20, H + 20], (B, 2)))
+    st["own_hs"][:, 0] = rng.uniform(0, 2 * np.pi, B)
+    st["goal"][:] = q(st["own_pos"] + rng.uniform(-30, 30, (B, 2)))
+    st["ipos"][:, : N // 2] = q(st["own_pos"][:, None, :] + rng.uniform(-40, 40, (B, N // 2, 2)))
+    st["ipos"][:, N // 2:] = q(rng.uniform(-20, [W + 20, H + 20], (B, N - N // 2, 2)))
+    st["ivel"][:] = rng.uniform(-2, 2, (B, N, 2))
+    lifted = envs[1].state
+    for k, v in st.items():
+        lifted[k][...] = v
+    for k in ("own_pos", "goal", "ipos"):
+        lifted[k][..., 1] += H2 - H
+    assert np.array_equal(lifted["own_pos"][:, 1].astype(np.float64) - (H2 - H), st["own_pos"][:, 1])
+    small, big = envs[0].raster(sprites.default_sprites()), envs[1].raster(sprites.default_sprites())
+    assert big.shape == (B, H2 // 4, W2 // 4)
+    assert np.array_equal(big[:, : H // 4, : W // 4], small)
+    assert (small != 255).sum() > 1000                          # there is a picture to compare
+
+
 def test_draw_order_later_sprites_on_top():
     e = _env(1)
     sp = sprites.default_sprites()
