@@ -308,12 +308,13 @@ __global__ void __launch_bounds__(128) step_own_kernel(const StepArgs a) {
 struct WarpScratch {
   uint32_t list[kTileRespawnCap];   // (lane of the env << 8 | intruder): the intruders that left the map in this step
   float2 pos[32];                   // the ownship the respawns keep their distance from (this step's position)
-  int tick[32];                     // tick of this step; -1: the env finished and was reset (its respawns are moot)
+  uint32_t tick[32];                // tick of this step (any uint32)
+  uint32_t moot;                    // bit e: env e finished and was reset, or is padding (its respawns are moot)
   int n_jobs;
 };
 struct BlockScratch {               // per block: the envs that finished under auto-reset (their N spawns, one warp per 32)
   int env[128];
-  int tick[128];                    // the tick of the step that finished the env
+  uint32_t tick[128];               // the tick of the step that finished the env
   float2 pos[128];                  // the ownship its new intruders keep their distance from (reset position)
   int count;
 };
@@ -556,7 +557,9 @@ __device__ __forceinline__ void finish_tile(const StepArgs& a, const int tile, c
   }
   if constexpr (PRE) {                                             // for the spawn phase (before a reset replaces pos)
     ws->pos[lane] = pos;
-    ws->tick[lane] = (has_env && !(done && a.auto_reset)) ? cnt.z : -1;
+    ws->tick[lane] = (uint32_t)cnt.z;
+    const uint32_t moot = __ballot_sync(FULL, !has_env || (done && a.auto_reset));
+    if (lane == 0) ws->moot = moot;
   }
 
   if constexpr (!TAPE) {
@@ -633,14 +636,14 @@ __device__ __forceinline__ void finish_tile(const StepArgs& a, const int tile, c
       reset_ownship<TAPE>(c, d, pos, hs, vel);
       if (reset_slot >= 0) {                                          // (the spawn phase reads them from shared memory)
         bs->pos[reset_slot] = pos;
-        bs->tick[reset_slot] = cnt.z;
+        bs->tick[reset_slot] = (uint32_t)cnt.z;
       }
     }
     cnt.w += 1;
     store_own_reset<FAITH>(a, me, pos, hs, vel, goal, cnt);
   }
   if (has_env) {
-    cnt.z += 1;                                                     // Philox tick; also flips the current position plane
+    cnt.z = (int)((uint32_t)cnt.z + 1u);                            // Philox tick (a uint32 that wraps); also flips the plane
     s.counters[me] = cnt;
     if constexpr (TAPE) a.cursor[me] = d.cur;
   }
@@ -670,13 +673,13 @@ __device__ __forceinline__ void spawn_phase(const StepArgs& a, const int tile, c
     for (int at = lane; at < n_resp; at += 32) {
       const uint32_t rec = ws->list[at];
       const int e = (int)(rec >> 8), i = (int)(rec & 0xffu);
-      const int tick = ws->tick[e];
-      if (tick < 0) continue;                               // the env finished and was reset: all its intruders are new anyway
+      if ((ws->moot >> e) & 1u) continue;                   // the env finished and was reset: all its intruders are new anyway
+      const uint32_t tick = ws->tick[e];
       const size_t env = (size_t)tile * 32 + e;
       const float2 own = ws->pos[e];
       d.env = a.env_id0 + (uint32_t)env;
-      d.tick = (uint32_t)tick;
-      const bool is64 = spawn_store<FAITH, false>(a, d, (uint32_t)i, env, i, (tick & 1) ^ 1, own.x, own.y,   // (the plane this step wrote)
+      d.tick = tick;
+      const bool is64 = spawn_store<FAITH, false>(a, d, (uint32_t)i, env, i, (int)(tick & 1u) ^ 1, own.x, own.y,   // (the plane this step wrote)
                                                   obs_intruder_base<FAITH>(a, env));
       if constexpr (FAITH) {
         if (is64) atomicOr(&s.dflag[flag_index(s, env, i >> 5)], 1u << (i & 31));
@@ -694,10 +697,10 @@ __device__ __forceinline__ void spawn_phase(const StepArgs& a, const int tile, c
   for (int job = wib; job < total; job += 4) {
     const size_t env = (size_t)bs->env[job / rounds];
     const int r = job % rounds;
-    const int tick = bs->tick[job / rounds];                // the tick of the step that finished the env
+    const uint32_t tick = bs->tick[job / rounds];           // the tick of the step that finished the env
     d.env = a.env_id0 + (uint32_t)env;
-    d.tick = (uint32_t)tick;
-    spawn_reset_word<FAITH>(a, d, env, r, lane, (tick & 1) ^ 1, bs->pos[job / rounds]);   // (the plane this step wrote)
+    d.tick = tick;
+    spawn_reset_word<FAITH>(a, d, env, r, lane, (int)(tick & 1u) ^ 1, bs->pos[job / rounds]);   // (the plane this step wrote)
   }
 }
 
@@ -847,6 +850,15 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? kFaithMinBlocks : 1) ste
     if (full) {
       // ---- all 8 intruders at once, straight-line
       fast_done = true;
+      // (the discard below) lane 8k's line of the plane just read is dead after the loads only if no real env of lanes
+      // 8k .. 8k+7 is on the other plane; settled here, before the loads, so that the masks and the loaded data are
+      // never live together (64 registers, as without the test)
+      bool discard = false;
+      if (a.auto_reset) {
+        const uint32_t odd = __ballot_sync(FULL, has_env && par), even = __ballot_sync(FULL, has_env && !par);
+        const uint32_t line = 0xffu << (lane & 24);
+        discard = (lane & 7) == 0 && !((odd & line) && (even & line));
+      }
       float4 p[kChunkUnits], np[kChunkUnits];
 #ifdef GCA_PHASE_TIMING
       const long long lat_t0 = clock64();
@@ -899,8 +911,10 @@ __global__ void __launch_bounds__(kWarpsB * 32, FAITH ? kFaithMinBlocks : 1) ste
       // DRAM (44.9 -> 43.3 us per step).  Lanes 0, 8, 16, 24 each discard the 128 bytes
       // that they and their 7 neighbours loaded; every (tile, unit) line is read by this warp only; the address
       // carries a dependency on the loaded data so that the discard cannot overtake the loads.  The plane is written in
-      // full by the next step (stream + spawn phase) before anything reads it again.
-      if (a.auto_reset && (lane & 7) == 0) {
+      // full by the next step (stream + spawn phase) before anything reads it again.  A line is dead only when every
+      // real env of its 8 read it: an env on the other plane (a masked reset or set_state moved its tick) has just
+      // stored its advanced positions into that very line.  (Padding lanes store nothing.)
+      if (discard) {
 #pragma unroll
         for (int g = 0; g < kChunkUnits; ++g) {
           const uint8_t* q = psrc + g * 512 + ((__float_as_uint(np[g].x) | __float_as_uint(np[g].w)) & 0u);
@@ -1088,7 +1102,7 @@ __global__ void __launch_bounds__(128) reset_kernel(const StepArgs a) {
   reset_envs_warp<FAITH, TAPE>(a, env0, lane, selected, nxt, d, pos, hs, vel, goal);
   if (selected) {
     store_own_reset<FAITH>(a, me, pos, hs, vel, goal, cnt);
-    cnt.z += 1;
+    cnt.z = (int)((uint32_t)cnt.z + 1u);
     s.counters[me] = cnt;
     if constexpr (TAPE) a.cursor[me] = d.cur;
     if (a.done) a.done[me] = 0;

@@ -139,7 +139,8 @@ typedef struct gca_host_state {
   double* goal;              /* [B][2]   :93 */
   int32_t* no_conflict;      /* [B]      :96 */
   int32_t* ep_steps;         /* [B]      steps since reset (StackEnv :118; TimeLimit) */
-  uint32_t* tick;            /* [B]      Philox tick: +1 per step and per explicit reset of that env */
+  uint32_t* tick;            /* [B]      Philox tick: +1 per step and per explicit reset of that env; any uint32,
+                                wraps from 2^32 - 1 to 0; tick & 1 picks the env's current position plane */
   double* ipos;              /* [B][N][2] intruder positions (f32-valued unless flagged) */
   uint8_t* ipos_is_f64;      /* [B][N]   position dtype is f64 (retried spawn, Q3) */
   float* ivel;               /* [B][N][2] :276 */
