@@ -76,6 +76,51 @@ def assert_state_equal(got, want, what="", skip=("ep_steps",), rows=None):
                 what, k, bad[:4].tolist(), a[tuple(bad[0])], b[tuple(bad[0])]))
 
 
+class ShardedOracle(object):
+    """The oracle over a whole batch, split into contiguous env ranges (bench.oracle_shards): one OracleEnv per host
+    thread, each with the env_id0 of its first env, so every env draws what the device's env of that global id draws.
+    ctypes releases the GIL, so the shards step in parallel.  Outputs and state are concatenated on demand."""
+
+    def __init__(self, cfg, B, N, seed, env_id0=0, f32_positions=True):
+        from concurrent.futures import ThreadPoolExecutor
+        from oracle import oracle as orc
+        threads = min(os.cpu_count() or 1, B)
+        self.bounds = [(int(r[0]), int(r[-1]) + 1) for r in np.array_split(np.arange(B), threads)]
+        self.shards = [orc.OracleEnv(cfg, hi - lo, N, draws=1, trig=orc.TRIG_SHARED, seed=seed, env_id0=env_id0 + lo,
+                                     f32_positions=f32_positions, auto_reset=True) for lo, hi in self.bounds]
+        self.pool = ThreadPoolExecutor(threads)
+        self.cfg, self.B, self.N, self.D = cfg, B, N, self.shards[0].D
+
+    def _each(self, fn):
+        list(self.pool.map(fn, range(len(self.shards))))
+
+    def reset(self):
+        self._each(lambda i: self.shards[i].reset())
+        return self.obs
+
+    def step(self, actions):
+        """actions: [B, 2] f64 (continuous) or [B] codes (discrete)."""
+        self._each(lambda i: self.shards[i].step(actions[self.bounds[i][0]:self.bounds[i][1]]))
+
+    def _cat(self, name):
+        return np.concatenate([getattr(s, name) for s in self.shards])
+
+    obs = property(lambda self: self._cat("obs"))
+    reward = property(lambda self: self._cat("reward"))
+    done = property(lambda self: self._cat("done"))
+    info = property(lambda self: self._cat("info"))
+    achieved = property(lambda self: self._cat("achieved"))
+    desired = property(lambda self: self._cat("desired"))
+    nearest = property(lambda self: self._cat("nearest"))
+
+    @property
+    def state(self):
+        return {k: np.concatenate([s.state[k] for s in self.shards]) for k in self.shards[0].state}
+
+    def close(self):
+        self.pool.shutdown()
+
+
 def golden_actions(variant_key, g):
     """[traces][T][2] action array of a golden file in the form the batched API takes:
     int codes in column 0 for the discrete kinds (the MCTS env's (a0, a1) tuple is a0*3+a1)."""
